@@ -9,13 +9,15 @@ One timed region is one ``tar_NB_attack(iters=K)`` call -- EXACTLY K steps: the 
 K-step loop.  The region is repeated ``--repeats`` times (L2 flushed before each); ``value`` is the
 median (min / max reported), each repeat the max over ranks.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU); every rank attacks its own 16 blocks (weak
 scaling, no data-path collective) and the per-class counters are all-reduced over NCCL afterwards.
 ``--impl reference`` times the UNMODIFIED reference (its own ``torchattacks.tar_NB_attack`` over its
 own ``pointnet2_sem_seg.get_model``, imported from oracle/_ref, see oracle/build_ref.py) on the host
 cores at the full B=16; if oracle/_ref is absent it falls back to the oracle port and says so.
+``--dump-outputs DIR`` writes what the last timed attack returned as ``DIR/adv.npy`` (float32 [B,9,N], the global batch
+in rank order): the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -118,6 +120,13 @@ def emit(line):
         os.write(_JSON_FD, data)
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each array of ``arrays`` as ``out_dir/<name>.npy`` in float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def make_inputs(B, seed=0):
     from pointsecguard_b200 import synthetic as syn
     x, labels = syn.make_painted_blocks(B, N_POINTS, seed)
@@ -130,7 +139,8 @@ def make_inputs(B, seed=0):
 # --------------------------------------------------------------------------------------------------
 def cpu_reference(steps, warmup_steps):
     """Times ``steps`` iterations of the reference's own tar_NB_attack on the full 16-block batch on all host threads,
-    after one warm-up attack of ``warmup_steps`` iterations.  Returns (steps/s, cores, kind, sample string, seconds).
+    after one warm-up attack of ``warmup_steps`` iterations.  Returns (steps/s, cores, kind, sample string, seconds,
+    the timed attack's perturbed blocks).
 
     The reference class handles a batch by reading ``labels[0]`` / ``outputs[0]`` (target.py:26,36): it runs the forward
     and the backward of all 16 blocks (the full cost of a 16-block step) with a [N] mask, which is what is timed; per-block
@@ -161,24 +171,25 @@ def cpu_reference(steps, warmup_steps):
     if warmup_steps > 0:
         run(warmup_steps)
     t0 = time.perf_counter()
-    run(steps)
+    adv = run(steps)
     dt = time.perf_counter() - t0
     sps = steps / dt
     sample = (f"tar-NB SSG, all 16 blocks x {steps} iterations (+ a warm-up attack of {warmup_steps}) on {cores} threads, "
               f"{dt:.1f} s; {who}")
-    return sps, cores, kind, sample, dt
+    return sps, cores, kind, sample, dt, adv
 
 
 def run_reference(args, rank):
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 48))
-    sps, cores, kind, sample, dt = cpu_reference(steps, max(0, min(args.warmup, 5)))
+    sps, cores, kind, sample, dt, adv = cpu_reference(args.steps, max(0, min(args.warmup, 5)))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"adv": adv.detach().numpy()})
     line = {
         "impl": "reference", "metric": METRIC, "value": sps, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": 1000.0 / sps, "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": config_dict(),
-        "timed_steps": steps, "timed_seconds": dt,
+        "timed_steps": args.steps, "timed_seconds": dt,
         "cpu_baseline": {"value": sps, "unit": UNIT, "cores": cores, "kind": kind, "sample": sample},
         "e2e": {"value": sps, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
@@ -328,6 +339,14 @@ def run_native(args, rank, world, local_rank):
     h2d = x_pin.numel() * 4 / K
     d2h = adv_host.numel() * 4 / K
     same_as_resident = bool(torch.equal(adv_host, adv.cpu()))
+    if args.dump_outputs:
+        out = adv.contiguous()
+        if world > 1:
+            full = torch.empty((world * out.shape[0],) + tuple(out.shape[1:]), dtype=out.dtype, device=dev)
+            dist.all_gather_into_tensor(full, out)
+            out = full
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"adv": out.cpu().numpy()})
 
     # ---- metrics + the only collective: per-class counters all-reduced over NCCL (timed on its own) ----
     torch.manual_seed(1)
@@ -442,7 +461,7 @@ def run_native(args, rank, world, local_rank):
         if args.no_cpu or world > 1:          # the CPU leg runs on rank 0 at N = 1 only
             cpu = None
         else:
-            sps, cores, kind, sample, _ = cpu_reference(5, 1)
+            sps, cores, kind, sample, _, _ = cpu_reference(5, 1)
             cpu = {"value": sps, "unit": UNIT, "cores": cores, "kind": kind, "sample": sample}
         line = {
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
@@ -622,7 +641,11 @@ def main():
     ap.add_argument("--mlp", default=os.environ.get("PSG_MLP", "tf32"), choices=["fp32", "tf32"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-parity", action="store_true", help="skip the fp32 parity-mode leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the perturbed blocks of the last timed attack to DIR/adv.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global _JSON_FD
     sys.stdout.flush()
     _JSON_FD = os.dup(1)
