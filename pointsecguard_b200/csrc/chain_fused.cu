@@ -692,7 +692,6 @@ __global__ void __launch_bounds__(NG * 128 + 64, 1) tile_kernel(const __grid_con
 }
 
 int g_sms = 0;
-bool g_use_clusters = true;
 long long *g_trace = nullptr;
 int g_dbg = 0;
 int g_trace_cap = 0, g_trace_n = 0;
@@ -753,14 +752,12 @@ int launch_tile(const TileArgs &a, int grid, size_t smem, cudaStream_t st)
     return PSG_OK;
 }
 
-bool g_use_ts = true;
-
 // A-operand-in-tensor-memory mode: row-local chains whose only refill is the interpolation (fp1 + head).  The operand
 // region needs whole 32-column stores and, with the accumulator, has to fit the 512 TMEM columns NG times.
 bool ts_eligible(const Builder &b, int ng)
 {
     const TileArgs &a = b.a;
-    if (!g_use_ts || b.amax_cols % 32) return false;
+    if (b.amax_cols % 32) return false;
     for (int o = 0; o < a.nops; ++o) {
         const TileOp &op = a.ops[o];
         if (op.pre != PRE_NONE && op.pre != PRE_FP) return false;
@@ -786,7 +783,7 @@ int launch_program(Builder &b, long long rows, cudaStream_t st)
     a.trace = psg_tile_trace_slot();
     a.abytes = b.amax_cols * 512;
     const int sms = (g_psg_sm_cap > 0 && g_psg_sm_cap < g_sms) ? g_psg_sm_cap : g_sms;
-    const int cs = g_use_clusters ? pick_cluster(a, a.ntiles, sms) : 1;
+    const int cs = pick_cluster(a, a.ntiles, sms);
     a.tcols = (int)pow2cols(b.nmax / cs);
     a.bias_floats = 0;
     for (int o = 0; o < a.nops; ++o) {
@@ -973,18 +970,16 @@ static bool fp_fits_whole(const PsgFpStream &f)
     for (int j = 0; j < f.nl; ++j) bias += (size_t)f.n[j] * 4;
     return (size_t)(f.C1 + f.C2) * 512 + 2 * 16 * 1024 + bias + 128 <= kSmemMax;
 }
-static bool g_fp_slabs = false;
-void psg_tile_set_fp_slabs(bool on) { g_fp_slabs = on; }
 
 bool psg_fp_streamable(const PsgFpStream &f, bool forward)
 {
     if (f.nl < 1 || f.nl > 3 || f.C1 % 16 || f.C2 % 16) return false;
     for (int j = 0; j < f.nl; ++j)
         if (f.n[j] % 32 || f.n[j] > 256) return false;
-    // Inputs wider than the operand buffer CAN be contracted in 256-column slabs (psg_fp_stream_fwd), but for the
-    // levels that need it (FP4: 1024 rows x 768 columns at B = 16) the per-layer GEMMs with their deep operand ring
-    // and 64 column-split CTAs measured faster (fp4 forward 45 us vs 95 us), so slabs stay opt-in ("fp_slabs").
-    return !forward || g_fp_slabs || fp_fits_whole(f);
+    // Forward inputs wider than the operand buffer run per layer: for the levels that have them (FP4: 1024 rows x 768
+    // columns at B = 16) the per-layer GEMMs with their deep operand ring and 64 column-split CTAs measured faster than
+    // a tile program contracting the input in 256-column slabs (fp4 forward 45 us vs 95 us).
+    return !forward || fp_fits_whole(f);
 }
 
 // [skip | interp] -> nl x (conv + folded BN + ReLU); last layer stored (it is the next level's
@@ -994,19 +989,8 @@ int psg_fp_stream_fwd(const PsgFpStream &f, cudaStream_t st)
     Builder b;
     int kprev = f.C1 + f.C2;
     for (int j = 0; j < f.nl; ++j) {
-        TileOp *o = nullptr;
-        if (j == 0 && !fp_fits_whole(f)) {
-            // the concatenated input is wider than the operand buffer: contract it in 256-column slabs, each slab
-            // refilled (skip rows / interpolation) while the accumulator carries over (FP4: 768 columns)
-            for (int k0 = 0; k0 < kprev; k0 += 256) {
-                const int ks = kprev - k0 < 256 ? kprev - k0 : 256;
-                o = b.add(f.wf[0], f.nwf[0], 0, k0 / 4, f.n[0], ks / 4, 0);
-                o->pre = PRE_FP; o->pre_a = k0 / 4; o->accumulate = k0 > 0 ? 1 : 0; o->epi = EPI_NONE;
-            }
-        } else {
-            o = b.add(f.wf[j], f.nwf[j], 0, 0, f.n[j], kprev / 4, 0);
-            if (j == 0) { o->pre = PRE_FP; o->pre_a = 0; }
-        }
+        TileOp *o = b.add(f.wf[j], f.nwf[j], 0, 0, f.n[j], kprev / 4, 0);
+        if (j == 0) { o->pre = PRE_FP; o->pre_a = 0; }
         o->bias = f.bias[j];
         if (j + 1 < f.nl) { o->epi = EPI_RELU; o->mglobal = f.m[j]; }
         else { o->epi = EPI_STORE; o->relu = 1; o->out = f.y_last; o->rm = f.y_last_rm; o->rm_stride = f.n[j]; }
@@ -1046,9 +1030,6 @@ int psg_fp_stream_bwd(const PsgFpStream &f, TView dy_last, TView dcat, float *dc
     return launch_program(b, f.rows, st);
 }
 
-// thread-block clusters for the deep levels (on by default; the switch exists for A/B measurements)
-void psg_tile_use_clusters(bool on) { g_use_clusters = on; }
-void psg_tile_use_ts(bool on) { g_use_ts = on; }
 void psg_tile_set_dbg(int v) { g_dbg = v; }
 long long *psg_tile_trace_slot() { return (g_trace && g_trace_n < g_trace_cap) ? g_trace + (size_t)(g_trace_n++) * 2048 : nullptr; }
 void psg_tile_set_trace(long long *buf, int nlaunches) { g_trace = buf; g_trace_cap = nlaunches; g_trace_n = 0; }

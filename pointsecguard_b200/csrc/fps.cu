@@ -382,8 +382,6 @@ static int launch_fps_cluster(int ppt, const float *xyz, long long cloud_stride,
 // cluster path for 16384 < N <= 65536 (psg_set_option "fps_cluster"; off until verified on the GPU in this round)
 static int g_fps_cluster = 1;
 void psg_fps_use_cluster(int on) { g_fps_cluster = on; }
-static int g_fps_fat_min_p = 128;      // psg_set_option "fps_fat_min_p": problems from which the 256 x 16 variant is used at N <= 4096
-void psg_fps_fat_min_p(int p) { g_fps_fat_min_p = p > 0 ? p : 128; }
 
 size_t psg_fps_workspace_bytes(int P, int N)
 {
@@ -401,7 +399,8 @@ int psg_fps_launch(const float *xyz, long long cloud_stride, int nclouds, int P,
     if (N <= 2048) return launch_fps<512, 4, 0>(xyz, cloud_stride, nclouds, P, N, npoint, start, out_idx, out_xyz, st);
     // many problems in flight (attack geometry batches): fewer, fatter threads -- the per-round warp
     // overhead (REDUX, barrier, exchange) is amortised over 16 points and 4 CTAs share an SM
-    if (N <= 4096 && N > 2048 && P >= g_fps_fat_min_p)
+    // (from 128 problems on: moving the threshold measured no difference for the smaller geometry passes)
+    if (N <= 4096 && N > 2048 && P >= 128)
         return launch_fps<256, 16, 0>(xyz, cloud_stride, nclouds, P, N, npoint, start, out_idx, out_xyz, st);
     if (N <= 4096) return launch_fps<1024, 4, 0>(xyz, cloud_stride, nclouds, P, N, npoint, start, out_idx, out_xyz, st);
     // few problems of a medium cloud: a cluster per problem (all resident at once) beats one CTA walking 16 points per

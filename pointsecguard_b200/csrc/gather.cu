@@ -9,10 +9,6 @@
 //   * row-major index_points for the public op                 (pointnet_util.py:43-60)
 #include "psg_common.cuh"
 #include "psg_internal.h"
-#include "psg_segsum.cuh"
-
-int g_psg_segsum_fast = 1;      // psg_set_option "segsum_fast": 0 restores the generic kernel
-int g_psg_segsum_warp = 0;      // psg_set_option "segsum_warp" n: rows of 32..32n chunks go through the warp-per-row kernel (measured: no gain, DESIGN.md section 4)
 
 namespace {
 
@@ -527,15 +523,6 @@ cudaError_t launch_segsum_fast(bool interp, bool rm, unsigned grid, cudaStream_t
     return psg_launch_pdl(segsum_fast_kernel<LPR, false, false>, dim3(grid), dim3(256), 0, st, 1, src, rpp, wgt, offs, perm, M, R, P, nch, dst, accumulate, rmk, src_rm, rs, tail);
 }
 
-// the same sums with a warp per destination row (psg_segsum.cuh): rows of >= 32 chunks
-template <int NC>
-__global__ void __launch_bounds__(256) segsum_warp_kernel(const PsgSegsumArgs a)
-{
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    asm volatile("griddepcontrol.wait;" ::: "memory");          // launched with programmatic stream serialization
-    psg_segsum_warp<NC, false>(a, (long long)blockIdx.x * 8 + (threadIdx.x >> 5), (long long)gridDim.x * 8, threadIdx.x & 31);
-}
-
 // dst[row][c] (+)= src[row][c] over a column slice
 __global__ void copy_cols_kernel(TView src, TView dst, long long rows, int nch, int accumulate)
 {
@@ -677,16 +664,7 @@ int psg_segsum(TView src, long long src_rows_per_p, int div, const float *wgt, c
     TView rm = relu_mask ? *relu_mask : TView{nullptr, 0, 0};
     const int nch = (ncols + 3) / 4;
     cudaError_t err = cudaSuccess;
-    if (nch >= 32 && nch <= 32 * g_psg_segsum_warp) {
-        PsgSegsumArgs a;
-        a.src = src; a.rows_per_p = src_rows_per_p; a.div = div; a.wgt = wgt; a.offs = offs; a.perm = perm; a.M = M; a.R = R; a.P = P;
-        a.nch = nch; a.tail = ncols & 3; a.dst = dst; a.acc = accumulate; a.rmask = rm; a.rm = src_rm; a.rm_stride = rm_stride;
-        const unsigned grid = nblocks(P * R * 32, 256);
-        if (nch <= 32) err = psg_launch_pdl(segsum_warp_kernel<1>, dim3(grid), dim3(256), 0, st, 1, a);
-        else if (nch <= 64) err = psg_launch_pdl(segsum_warp_kernel<2>, dim3(grid), dim3(256), 0, st, 1, a);
-        else err = psg_launch_pdl(segsum_warp_kernel<4>, dim3(grid), dim3(256), 0, st, 1, a);
-    } else if (g_psg_segsum_fast && ((div == 3 && wgt) || (div == 1 && !wgt)) &&
-               src_rows_per_p < (1ll << 24) && (long long)M < (1ll << 30)) {
+    if (((div == 3 && wgt) || (div == 1 && !wgt)) && src_rows_per_p < (1ll << 24) && (long long)M < (1ll << 30)) {
         // the two real callers (interpolation backward, gather backward): specialised kernel, same sums
         const bool interp = div == 3, rmm = src_rm != nullptr;
         const int lpr = nch <= 4 ? 4 : nch <= 8 ? 8 : nch <= 16 ? 16 : nch <= 32 ? 32 : nch <= 64 ? 64 : 128;
@@ -694,8 +672,7 @@ int psg_segsum(TView src, long long src_rows_per_p, int div, const float *wgt, c
 #define PSG_SF(L) launch_segsum_fast<L>(interp, rmm, grid, st, src, src_rows_per_p, wgt, offs, perm, M, R, P, nch, dst, accumulate, rm, src_rm, rm_stride, ncols & 3)
         err = lpr == 4 ? PSG_SF(4) : lpr == 8 ? PSG_SF(8) : lpr == 16 ? PSG_SF(16) : lpr == 32 ? PSG_SF(32) : lpr == 64 ? PSG_SF(64) : PSG_SF(128);
 #undef PSG_SF
-    } else
-    if (nch <= 4)
+    } else if (nch <= 4)
         err = psg_launch_pdl(segsum_kernel<4>, dim3(nblocks(P * R * 4, 256)), dim3(256), 0, st, 1, src, src_rows_per_p, div, wgt,
                              offs, perm, M, R, P, nch, ncols & 3, dst, accumulate, rm, src_rm, rm_stride);
     else if (nch <= 8)

@@ -248,8 +248,9 @@ __global__ void __launch_bounds__(kThreads) gemm_tc_kernel(PsgGemmArgs g, int bn
     if (warp == 1) tc::tmem_dealloc(tmem, ncols);
 }
 
-int g_big_kb8 = 1;      // psg_set_option "gemm_two_ctas": 0 keeps one CTA per SM behind the full ring for large layers
-int g_nst_plain = 2, g_nst_x3 = 1, g_big_ctas = 148;      // ring depth of the many-tile layers, and what "many" means (measured: MSG B = 64 275 -> 295 steps/s, 3xTF32 mode 409 -> 536)
+// ring depth of the many-tile layers, and what "many" means: two CTAs per SM instead of one behind the full ring
+// (measured: MSG B = 64 275 -> 295 steps/s, 3xTF32 mode 409 -> 536)
+constexpr int kNstPlain = 2, kNstX3 = 1, kBigCtas = 148;
 
 template <int EPI, bool X3, int KB>
 int launch_kb(const PsgGemmArgs &g, int bn, cudaStream_t st)
@@ -271,8 +272,8 @@ int launch_kb(const PsgGemmArgs &g, int bn, cudaStream_t st)
     if (nst > kstages) nst = kstages;
     // many tiles and a long K loop: three stages per CTA so that TWO CTAs share an SM -- one's epilogue and prologue run
     // under the other's K loop (a single CTA behind the whole ring serialises them: MSG sa4, 256 row tiles x K = 512)
-    if (!X3 && KB == 8 && nst > g_nst_plain) nst = g_nst_plain;
-    if (X3 && g_big_kb8 && bn <= 64 && nst > g_nst_x3 && (long long)g.mtiles * ((g.nout_pad + bn - 1) / bn) > g_big_ctas) nst = g_nst_x3;
+    if (!X3 && KB == 8 && nst > kNstPlain) nst = kNstPlain;
+    if (X3 && bn <= 64 && nst > kNstX3 && (long long)g.mtiles * ((g.nout_pad + bn - 1) / bn) > kBigCtas) nst = kNstX3;
     const size_t smem = (size_t)nst * stage_bytes + 1024;
     dim3 grid((unsigned)g.mtiles, (unsigned)((g.nout_pad + bn - 1) / bn));
     // weights [K/4][Nw][4] as a tiled TMA source: boxes of kBlk planes x bn columns (K is a multiple of 16, i.e. of
@@ -296,7 +297,7 @@ int launch(const PsgGemmArgs &g, cudaStream_t st)
     if (X3) {
         // 3xTF32 stages hold A, A_lo, W_hi and W_lo: with 128-column tiles one CTA fills an SM.  Layers with far more
         // tiles than SMs take 64-column tiles and a two-stage ring instead, so that two CTAs overlap on every SM.
-        if (g_big_kb8 && bn > 64 && (long long)g.mtiles * ((g.nout_pad + bn - 1) / bn) > g_big_ctas) bn = 64;
+        if (bn > 64 && (long long)g.mtiles * ((g.nout_pad + bn - 1) / bn) > kBigCtas) bn = 64;
         return launch_kb<EPI, X3, 8>(g, bn, st);
     }
     // 32 KB activation stages by default (the producer's per-stage cost bounds the K loop); 16 KB stages x 3 when the
@@ -304,19 +305,11 @@ int launch(const PsgGemmArgs &g, cudaStream_t st)
     const long long ctas = (long long)g.mtiles * ((g.nout_pad + bn - 1) / bn);
     const int kstages16 = (g.k1chunks + 15) / 16 + (g.k2chunks + 15) / 16;
     const long long ring16 = (long long)(kstages16 < kRingBytes / (32768 + 16 * bn * 16) ? kstages16 : kRingBytes / (32768 + 16 * bn * 16)) * (32768 + 16 * bn * 16);
-    if (g_big_kb8 && ctas > g_big_ctas && ring16 > 112 * 1024) return launch_kb<EPI, false, 8>(g, bn, st);
+    if (ctas > kBigCtas && ring16 > 112 * 1024) return launch_kb<EPI, false, 8>(g, bn, st);
     return launch_kb<EPI, false, 16>(g, bn, st);
 }
 
 }  // namespace
-
-void psg_gemm_tc_two_ctas(int on) { g_big_kb8 = on; }
-void psg_gemm_tc_tune(int nst_plain, int nst_x3, int big_ctas)
-{
-    if (nst_plain > 0) g_nst_plain = nst_plain;
-    if (nst_x3 > 0) g_nst_x3 = nst_x3;
-    if (big_ctas > 0) g_big_ctas = big_ctas;
-}
 
 int psg_gemm_tc(const PsgGemmArgs &g, cudaStream_t st)
 {

@@ -25,16 +25,13 @@ long long g_psg_launch_count = 0;
 int g_psg_sm_cap = 0;
 // FP levels with fewer 128-row tiles than this run per layer: with a third of the SMs or fewer busy, 64 column-split
 // GEMM CTAs with a deep operand ring beat one cluster per tile (B = 16: fp3 as a tile program 1133 steps/s, per
-// layer 1153; psg_set_option "fp_min_tiles")
-static int g_fp_min_tiles = 48;
+// layer 1153)
+static const int kFpMinTiles = 48;
 // fused SA branches run on compacted neighbourhood rows (compact.cu); psg_set_option "sa_compact" 0 restores the padded layout
 static int g_sa_compact = 1;
-// the per-layer FP levels (fp4 / fp3 at B = 16) and the segmented sums around them run as ONE persistent kernel per
-// direction (deep.cu: phase list + grid barrier) instead of a launch per layer; psg_set_option "deep" 0 restores the launches
 // mode 2 (3xTF32): the narrow SA branches run as fused kernels too when their hi + lo weights and operand buffers fit
 // (psg_set_option "x3_fused" 0: every layer of mode 2 goes through the per-layer GEMM)
 static int g_x3_fused = 3;     // bit 0: the narrow SA branches, bit 1: fp1 + head
-static int g_deep = 0;      // bit 0: on; bit 1: the backward kernel starts with the segmented sum that feeds its first level (OFF by default: measured slower, DESIGN.md section 4)
 
 // ------------------------------------------------------------------------------------------------
 // per-kernel-family device timing (bench.py's live roofline measurement).  When enabled, every
@@ -43,11 +40,11 @@ static int g_deep = 0;      // bit 0: on; bit 1: the backward kernel starts with
 // ------------------------------------------------------------------------------------------------
 enum { PF_FPS, PF_BALL, PF_NN3, PF_CSR, PF_PACK, PF_GROUP, PF_GEMM_FWD, PF_MAXPOOL, PF_INTERP, PF_HEAD, PF_LOSS,
        PF_GEMM_BWD, PF_MAXPOOL_BWD, PF_SEGSUM, PF_COPY, PF_PGD, PF_SA_FWD, PF_SA_BWD, PF_FP_FWD, PF_FP_BWD, PF_HEAD_CHAIN,
-       PF_DEEP_FWD, PF_DEEP_BWD, PF_NCAT };
+       PF_NCAT };
 static const char *kProfNames[PF_NCAT] = {"fps", "ball_query", "three_nn", "csr_build", "pack", "group", "gemm_fwd",
                                           "maxpool", "interp", "head", "loss_grad", "gemm_bwd", "maxpool_bwd", "segsum",
                                           "copy_cols", "pgd_update", "sa_fused_fwd", "sa_fused_bwd", "fp_fused_fwd",
-                                          "fp_fused_bwd", "head_chain", "deep_fwd", "deep_bwd"};
+                                          "fp_fused_bwd", "head_chain"};
 namespace {
 struct ProfRec { cudaEvent_t a, b; int cat; };
 bool g_prof_on = false;
@@ -121,7 +118,7 @@ struct psg_mlp {
 // What remains is zero-mean rounding noise (std ~0.29 ulp per operand, the same as round-to-nearest would leave), which
 // averages over the K terms of a dot product instead of accumulating.
 static const double kTf32Comp = 3.45e-4;
-static double kX3AccComp = 6.6e-9;       // per column of contraction (psg_set_option "x3_acc_comp_e10": value x 1e-10, for A/B)
+static const double kX3AccComp = 6.6e-9;       // 3xTF32 accumulator truncation per column of contraction (psg_mlp_create)
 static inline float tf32_rna(double x)
 {
     float f = (float)x;
@@ -224,7 +221,6 @@ extern "C" void psg_mlp_destroy(psg_mlp *m)
 
 static int run_gemm(const PsgGemmArgs &g, int mode, cudaStream_t st)
 {
-    if (mode == 1 && psg_deep_recording()) return psg_deep_add_gemm(g);      // a phase of the deep kernel (deep.cu)
     return mode >= 1 ? psg_gemm_tc(g, st) : psg_gemm_simt(g, st);
 }
 
@@ -352,9 +348,6 @@ struct psg_net {
     float *H, *Z, *dZ;
     float *S[2]; size_t scratch_floats;
     float *Srm;            // row-major copy of the gradient rows a fused backward kernel hands to the segmented sum
-    unsigned *deep_ctr;    // grid-barrier counter + error word of the deep kernel (deep.cu)
-    unsigned deep_epoch;   // arrivals earlier launches left in deep_ctr[0]
-    bool deep_reset;       // the counter has not been zeroed since the workspace was bound
     bool bound;
     int last_t;
     // tcgen05 mode: fp1 + head run as one forward+backward kernel (chain_fused.cu); the loss is then
@@ -474,28 +467,11 @@ extern "C" int psg_set_option(const char *name, int value)
     if (!name) return PSG_EINVAL;
     if (!strcmp(name, "nn_grid")) { psg_three_nn_grid_mode(value); return PSG_OK; }
     if (!strcmp(name, "fps_cluster")) { psg_fps_use_cluster(value); return PSG_OK; }
-    if (!strcmp(name, "fps_fat_min_p")) { psg_fps_fat_min_p(value); return PSG_OK; }
-    if (!strcmp(name, "ts")) { psg_tile_use_ts(value != 0); return PSG_OK; }
-    if (!strcmp(name, "clusters")) { psg_tile_use_clusters(value != 0); return PSG_OK; }
-    if (!strcmp(name, "fp_min_tiles")) { g_fp_min_tiles = value; return PSG_OK; }
-    if (!strcmp(name, "fp_slabs")) { psg_tile_set_fp_slabs(value != 0); return PSG_OK; }
-    if (!strcmp(name, "sa_ng")) { psg_sa_force_ng(value); return PSG_OK; }
     if (!strcmp(name, "sa_compact")) { g_sa_compact = value != 0; return PSG_OK; }
-    if (!strcmp(name, "deep")) { g_deep = value; return PSG_OK; }
     if (!strcmp(name, "x3_fused")) { g_x3_fused = value; return PSG_OK; }
-    if (!strcmp(name, "x3_acc_comp_e10")) { kX3AccComp = value * 1e-10; return PSG_OK; }     // takes effect for layers created afterwards
-    if (!strcmp(name, "deep_bn_min")) { psg_deep_tune(value, 0); return PSG_OK; }
-    if (!strcmp(name, "deep_items")) { psg_deep_tune(0, value); return PSG_OK; }
     if (!strcmp(name, "stream_stages")) { psg_stream_tune(value, 0, 0); return PSG_OK; }
     if (!strcmp(name, "stream_stage_bytes")) { psg_stream_tune(0, value, 0); return PSG_OK; }
     if (!strcmp(name, "stream_rings")) { psg_stream_tune(0, 0, value); return PSG_OK; }
-    if (!strcmp(name, "gemm_nst_plain")) { psg_gemm_tc_tune(value, 0, 0); return PSG_OK; }
-    if (!strcmp(name, "gemm_nst_x3")) { psg_gemm_tc_tune(0, value, 0); return PSG_OK; }
-    if (!strcmp(name, "gemm_big_ctas")) { psg_gemm_tc_tune(0, 0, value); return PSG_OK; }
-    if (!strcmp(name, "gemm_two_ctas")) { psg_gemm_tc_two_ctas(value); return PSG_OK; }
-    if (!strcmp(name, "segsum_fast")) { g_psg_segsum_fast = value; return PSG_OK; }
-    if (!strcmp(name, "segsum_warp")) { g_psg_segsum_warp = value; return PSG_OK; }
-    if (!strcmp(name, "sa_grid_div")) { psg_sa_grid_div(value); return PSG_OK; }
     if (!strcmp(name, "dbg")) { psg_tile_set_dbg(value); return PSG_OK; }
     if (!strcmp(name, "sm_cap")) { g_psg_sm_cap = value > 0 ? value : 0; return PSG_OK; }
     return PSG_EINVAL;
@@ -589,7 +565,7 @@ static size_t plan(psg_net *n, int B, int N, int T, char *base)
         for (int j = 0; j < 3; ++j) F.m[j] = nullptr;
         if (f > 0) {
             PsgFpStream q = fp_stream_desc(n, f, 0, TView{nullptr, 0, 0});
-            F.streamed = psg_fp_streamable(q, true) && psg_fp_streamable(q, false) && (rows + 127) / 128 >= g_fp_min_tiles;
+            F.streamed = psg_fp_streamable(q, true) && psg_fp_streamable(q, false) && (rows + 127) / 128 >= kFpMinTiles;
             if (F.streamed)
                 for (int j = 0; j + 1 < F.nl; ++j) F.m[j] = bp.take<unsigned>(psg_sa_mask_words(rows, F.mlp[j]->npad));
         }
@@ -611,7 +587,6 @@ static size_t plan(psg_net *n, int B, int N, int T, char *base)
     n->S[0] = bp.take<float>(scratch);
     n->S[1] = bp.take<float>(scratch);
     n->Srm = bp.take<float>(scratch);
-    n->deep_ctr = bp.take<unsigned>(32);
     n->fps_ws = bp.take<char>(n->fps_ws_bytes ? n->fps_ws_bytes : 16);
     n->csr_ws = bp.take<char>(csr_scratch);
     n->grid_ws = N >= 2048 ? (void *)bp.take<char>(psg_ballgrid_workspace_bytes(B, N)) : nullptr;
@@ -637,7 +612,6 @@ extern "C" int psg_net_bind(psg_net *n, int B, int N, int T, void *ws, size_t ws
     if (ws_bytes < need) return PSG_EWORKSPACE;
     plan(n, B, N, T, (char *)ws);
     n->B = B; n->N = N; n->T = T; n->bound = true; n->last_t = -1;
-    n->deep_reset = true; n->deep_epoch = 0;
     return PSG_OK;
 }
 
@@ -646,19 +620,6 @@ extern "C" int psg_net_bind(psg_net *n, int B, int N, int T, void *ws, size_t ws
         int rc__ = (expr);                \
         if (rc__ != PSG_OK) return rc__;  \
     } while (0)
-
-// launch what the deep recorder holds (nothing if it is not recording)
-static int deep_flush(psg_net *n, int cat, cudaStream_t st)
-{
-    if (!psg_deep_recording()) return PSG_OK;
-    if (psg_deep_phases() == 0) { psg_deep_cancel(); return PSG_OK; }
-    if (n->deep_reset) {
-        if (cudaMemsetAsync(n->deep_ctr, 0, 32 * sizeof(unsigned), st) != cudaSuccess) return PSG_ECUDA;
-        n->deep_reset = false; n->deep_epoch = 0;
-    }
-    PSG_RUN(cat, psg_deep_flush(n->deep_ctr, &n->deep_epoch, st));
-    return PSG_OK;
-}
 
 extern "C" int psg_net_set_input(psg_net *n, const float *x, int64_t sb, int64_t sc, int64_t sn, psg_stream_t stream)
 {
@@ -896,15 +857,10 @@ extern "C" int psg_net_forward(psg_net *n, int t, float *logp, float *l4_points,
     const bool fuse_head = head_fused_now(n);
     n->z_valid = false;
     n->loss.set = false;
-    psg_deep_cancel();
     for (int f = 3; f >= 0; --f) {
         FpLevel &F = n->fp[f];
         const int Nf = n->npts[f], Nc = n->npts[f + 1];
         const long long rows = (long long)B * Nf;
-        const bool per_layer = !(f == 0 && fuse_head) && !(mode == 1 && F.streamed);
-        // consecutive per-layer levels (few rows: the deep levels) are recorded and run as one persistent kernel
-        if (!per_layer || rows > 8192) PSG_TRY(deep_flush(n, PF_DEEP_FWD, st));
-        else if (mode == 1 && (g_deep & 1) && !psg_deep_recording()) psg_deep_begin();
         if (f == 0 && fuse_head) {
             // fp1 + head as one kernel; when nobody asked for the log-probabilities the whole chain is
             // deferred to psg_net_backward, which runs it forward AND backward in one pass
@@ -922,11 +878,6 @@ extern "C" int psg_net_forward(psg_net *n, int t, float *logp, float *l4_points,
             up = F.Y[F.nl - 1]; upw = F.mlp[F.nl - 1]->npad;
             continue;
         }
-        if (psg_deep_recording() && psg_deep_phases() + 1 + F.nl > PSG_DEEP_MAX_PHASES) { PSG_TRY(deep_flush(n, PF_DEEP_FWD, st)); psg_deep_begin(); }
-        if (psg_deep_recording())
-            PSG_TRY(psg_deep_add_interp(tv(up, upw), Nc, F.nn_idx + (size_t)t * B * Nf * 3, F.nn_w + (size_t)t * B * Nf * 3, B, Nf,
-                                        F.C2 / 4, tv(F.I, F.C2)));
-        else
         PSG_RUN(PF_INTERP, psg_interp(tv(up, upw), Nc, F.nn_idx + (size_t)t * B * Nf * 3, F.nn_w + (size_t)t * B * Nf * 3, B, Nf,
                            F.C2 / 4, tv(F.I, F.C2), st));
         TView a1 = F.C1 ? tv(n->feats[f], n->wfeat[f]) : tv(F.I, F.C2);
@@ -939,7 +890,6 @@ extern "C" int psg_net_forward(psg_net *n, int t, float *logp, float *l4_points,
         }
         up = F.Y[F.nl - 1]; upw = F.mlp[F.nl - 1]->npad;
     }
-    PSG_TRY(deep_flush(n, PF_DEEP_FWD, st));
     const long long rows0 = (long long)B * n->N;
     if (!fuse_head) {
         PSG_RUN(PF_GEMM_FWD, mlp_fwd(n->conv1, tv(up, upw), upw / 4, none, 0, rows0, tv(n->H, n->conv1->npad), 1, mode, st));
@@ -1017,22 +967,10 @@ extern "C" int psg_net_backward(psg_net *n, int t, float *grad_x, psg_stream_t s
     // ---- head + feature propagation, fine to coarse ----
     TView top = tv(n->dZ, n->conv2->npad);
     int top_buf = -1;
-    psg_deep_cancel();
-    const bool deep_ok = n->mode == 1 && (g_deep & 1) && !n->xyz_grad;
-    // levels that run per layer and hold few rows: their dgrad GEMMs and the segmented sums around them become phases
-    // of one persistent kernel (deep.cu)
-    auto deep_level = [&](int f) {
-        return deep_ok && f >= 1 && f <= 3 && !n->fp[f].streamed && (long long)B * n->npts[f] <= 8192;
-    };
     for (int f = 0; f <= 3; ++f) {
         FpLevel &F = n->fp[f];
         const int Nf = n->npts[f], Nc = n->npts[f + 1];
         const long long rows = (long long)B * Nf;
-        if (!deep_level(f)) PSG_TRY(deep_flush(n, PF_DEEP_BWD, st));
-        else {
-            if (psg_deep_recording() && psg_deep_phases() + F.nl + 1 > PSG_DEEP_MAX_PHASES) PSG_TRY(deep_flush(n, PF_DEEP_BWD, st));
-            if (!psg_deep_recording()) psg_deep_begin();
-        }
         psg_mlp *mlps[5]; float *Ys[5]; int nl = 0;
         for (int j = 0; j < F.nl; ++j) { mlps[nl] = F.mlp[j]; Ys[nl] = F.Y[j]; ++nl; }
         if (f == 0) { mlps[nl] = n->conv1; Ys[nl] = n->H; ++nl; mlps[nl] = n->conv2; Ys[nl] = n->Z; ++nl; }
@@ -1061,10 +999,10 @@ extern "C" int psg_net_backward(psg_net *n, int t, float *grad_x, psg_stream_t s
             TView dsk = tv(n->dfeat[f], n->wfeat[f]);
             PSG_TRY(chain_bwd(n, mlps, Ys, nl, rows, top, top_buf, &cat_buf, st, &dsk, F.C1));
             skip_done = true;
-        } else
-        PSG_TRY(chain_bwd(n, mlps, Ys, nl, rows, top, top_buf, &cat_buf, st));
+        } else {
+            PSG_TRY(chain_bwd(n, mlps, Ys, nl, rows, top, top_buf, &cat_buf, st));
+        }
         const int catw = F.C1 + F.C2;
-        if (F.C1 && !skip_done) PSG_TRY(deep_flush(n, PF_DEEP_BWD, st));
         if (F.C1 && !skip_done) PSG_RUN(PF_COPY, psg_copy_cols(tv(n->S[cat_buf], catw), tv(n->dfeat[f], n->wfeat[f]), rows, F.C1, 0, st));
         // interpolation backward: scatter the three weighted copies to the coarse level, in CSR order
         const size_t go = (size_t)t * B;
@@ -1077,32 +1015,21 @@ extern "C" int psg_net_backward(psg_net *n, int t, float *grad_x, psg_stream_t s
                                                    F.csr_off + go * (Nc + 1), F.csr_perm + go * Nf * 3, B, Nf, n->dxyz[f],
                                                    n->dxyz[f + 1], n->xyz_tmp, st));
         }
-        // the segmented sum that feeds a deep level opens that level's kernel
-        if (!psg_deep_recording() && f < 3 && deep_level(f + 1) && (g_deep & 2)) psg_deep_begin();
-        if (psg_deep_recording() && !psg_deep_can_segsum(F.C2)) PSG_TRY(deep_flush(n, PF_DEEP_BWD, st));
         if (f < 3) {
             FpLevel &C = n->fp[f + 1];
             const int cw = C.mlp[C.nl - 1]->npad;
             const int dst_buf = cat_buf ^ 1;
             TView dst = tv(n->S[dst_buf], cw);
             TView mk = tv(C.Y[C.nl - 1], cw);
-            if (psg_deep_recording())
-                PSG_TRY(psg_deep_add_segsum(tv(n->S[cat_buf], catw, F.C1), Nf, 3, F.nn_w + go * Nf * 3, F.csr_off + go * (Nc + 1),
-                                            F.csr_perm + go * Nf * 3, Nf * 3, Nc, B, F.C2, dst, 0, &mk, rm_src, rm_stride));
-            else
             PSG_RUN(PF_SEGSUM, psg_segsum(tv(n->S[cat_buf], catw, F.C1), Nf, 3, F.nn_w + go * Nf * 3, F.csr_off + go * (Nc + 1),
-                               F.csr_perm + go * Nf * 3, Nf * 3, Nc, B, F.C2, dst, 0, &mk, rm_src, rm_stride, st));
+                                          F.csr_perm + go * Nf * 3, Nf * 3, Nc, B, F.C2, dst, 0, &mk, rm_src, rm_stride, st));
             top = dst; top_buf = dst_buf;
         } else {
-            if (psg_deep_recording())
-                PSG_TRY(psg_deep_add_segsum(tv(n->S[cat_buf], catw, F.C1), Nf, 3, F.nn_w + go * Nf * 3, F.csr_off + go * (Nc + 1),
-                                            F.csr_perm + go * Nf * 3, Nf * 3, Nc, B, F.C2, tv(n->dfeat[4], n->wfeat[4]), 0, nullptr, rm_src, rm_stride));
-            else
             PSG_RUN(PF_SEGSUM, psg_segsum(tv(n->S[cat_buf], catw, F.C1), Nf, 3, F.nn_w + go * Nf * 3, F.csr_off + go * (Nc + 1),
-                               F.csr_perm + go * Nf * 3, Nf * 3, Nc, B, F.C2, tv(n->dfeat[4], n->wfeat[4]), 0, nullptr, rm_src, rm_stride, st));
+                                          F.csr_perm + go * Nf * 3, Nf * 3, Nc, B, F.C2, tv(n->dfeat[4], n->wfeat[4]), 0, nullptr,
+                                          rm_src, rm_stride, st));
         }
     }
-    PSG_TRY(deep_flush(n, PF_DEEP_BWD, st));
     // ---- set abstraction, coarse to fine ----
     for (int l = 4; l >= 1; --l) {
         SaLevel &L = n->sa[l - 1];

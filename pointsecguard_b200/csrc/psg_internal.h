@@ -35,7 +35,6 @@ int psg_scene_gather_k(const double *pts, int ld, int label_col, const int *sel,
 
 // fps.cu
 void psg_fps_use_cluster(int on);
-void psg_fps_fat_min_p(int p);
 size_t psg_fps_workspace_bytes(int P, int N);
 int psg_fps_launch(const float *xyz, long long cloud_stride, int nclouds, int P, int N, int npoint,
                    const int *start, int *out_idx, float *out_xyz, void *ws, size_t ws_bytes, cudaStream_t st);
@@ -70,7 +69,6 @@ int psg_csr_build(const int *keys, long long P, int M, int R, int grp, int *offs
 int psg_segsum(TView src, long long src_rows_per_p, int div, const float *wgt, const int *offs, const int *perm,
                int M, int R, long long P, int ncols, TView dst, int accumulate, const TView *relu_mask, const float *src_rm,
                int rm_stride, cudaStream_t st);
-extern int g_psg_segsum_warp, g_psg_segsum_fast;
 int psg_copy_cols(TView src, TView dst, long long rows, int ncols, int accumulate, cudaStream_t st);
 int psg_index_points_rm(const float *pts, const long long *idx, int B, int N, int C, long long M, float *out,
                         cudaStream_t st);
@@ -82,22 +80,6 @@ void psg_stream_tune(int stages, int stage_bytes, int rings);
 // gemm_simt.cu / gemm_tc.cu
 int psg_gemm_simt(const PsgGemmArgs &g, cudaStream_t st);
 int psg_gemm_tc(const PsgGemmArgs &g, cudaStream_t st);
-void psg_gemm_tc_two_ctas(int on);
-void psg_gemm_tc_tune(int nst_plain, int nst_x3, int big_ctas);
-// deep.cu: the per-layer FP levels as one persistent kernel -- a recorder collects the phases, flush launches them
-#define PSG_DEEP_MAX_PHASES 10
-void psg_deep_begin();
-void psg_deep_tune(int bn_min, int items_min);
-bool psg_deep_recording();
-int psg_deep_phases();
-void psg_deep_cancel();
-bool psg_deep_can_gemm(const PsgGemmArgs &g);
-int psg_deep_add_gemm(const PsgGemmArgs &g);
-int psg_deep_add_interp(TView feats, int S, const int *idx, const float *w, long long P, int N, int nch, TView out);
-bool psg_deep_can_segsum(int ncols);
-int psg_deep_add_segsum(TView src, long long src_rows_per_p, int div, const float *wgt, const int *offs, const int *perm, int M, int R,
-                        long long P, int ncols, TView dst, int accumulate, const TView *relu_mask, const float *src_rm, int rm_stride);
-int psg_deep_flush(unsigned *ctr, unsigned *epoch, cudaStream_t st);
 // sa_fused.cu: one set-abstraction branch (gather -> 3 layers -> neighbourhood max) per kernel
 // compact.cu: compacted neighbourhood rows (real ball-query hits only) of one fused SA branch
 struct PsgCompact {
@@ -133,8 +115,6 @@ struct PsgSaFused {
 };
 bool psg_sa_fusable(int K, int gpad, int n0, int n1, int n2);
 bool psg_sa_fusable_x3(int K, int gpad, int n0, int n1, int n2);
-void psg_sa_grid_div(int d);       // A/B switch: grid of the compacted-row kernels = padded tiles / d (default 1)
-void psg_sa_force_ng(int ng);      // A/B switch: tiles in flight per CTA of the fused SA kernels (0 = automatic)
 size_t psg_sa_mask_words(long long rows, int n);
 int psg_sa_fused_fwd(const PsgSaFused &f, cudaStream_t st);
 int psg_sa_fused_bwd(const PsgSaFused &f, TView dout, TView dG, int gcols, float *dG_rm, int rm_only, cudaStream_t st);
@@ -171,10 +151,7 @@ struct PsgFpStream {
 bool psg_fp_streamable(const PsgFpStream &f, bool forward);
 int psg_fp_stream_fwd(const PsgFpStream &f, cudaStream_t st);
 int psg_fp_stream_bwd(const PsgFpStream &f, TView dy_last, TView dcat, float *dcat_rm, TView dskip, cudaStream_t st);
-void psg_tile_use_clusters(bool on);
-void psg_tile_use_ts(bool on);     // A operand of the row-local chains in tensor memory (default on)
 void psg_tile_set_dbg(int v);
-void psg_tile_set_fp_slabs(bool on);
 long long *psg_tile_trace_slot();   // next [4][512] block of the debug trace buffer, or null
 void psg_tile_set_trace(long long *buf, int nlaunches);
 // geomgrad.cu: gradient w.r.t. coordinates through grouping and interpolation weights

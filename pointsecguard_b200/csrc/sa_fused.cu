@@ -725,12 +725,11 @@ void (*bwd_kern_cp(int ng))(SaBwdArgs)
 // (fewer CTAs: fewer prologues, weights loaded fewer times).  Decisions are cached per configuration.
 struct Pick { int ng, occ; };
 template <class KernOf, class SmemOf>
-Pick pick_ng(KernOf kern_of, SmemOf smem_of, int gc, int ng_forced = 0)
+Pick pick_ng(KernOf kern_of, SmemOf smem_of, int gc)
 {
     Pick best{0, 0};
     int best_tiles = 0;
     for (int ng = 1; ng <= 4; ++ng) {
-        if (ng_forced && ng != ng_forced) continue;
         const size_t sm = smem_of(ng);
         if (sm > kSmemPerCtaMax || ng * gc > 512) break;
         const int occ = ctas_per_sm(kern_of(ng), ng * 160, sm, (int)pow2cols(ng * gc));
@@ -743,18 +742,7 @@ struct PickKey { int dir, K, gpad, n0, n1, n2, cap, dev; };
 struct PickEnt { PickKey k; Pick p; };
 PickEnt g_picks[128];
 int g_npicks = 0;
-int g_ng_forced = 0;
-// compacted rows: only the device knows the tile count.  The grid is sized for padded tiles / g_grid_div; 1 = as if nothing
-// compacted (CTAs without a tile leave after the prologue), 3 = the S3DIS-density guess of the first version, which left
-// SA2 (rows / 2, not / 3.6) on 86 of 148 SMs for two rounds of tiles
-int g_grid_div = 1;
 
-}  // namespace
-
-void psg_sa_force_ng(int ng) { g_ng_forced = ng; g_npicks = 0; }
-void psg_sa_grid_div(int d) { g_grid_div = d < 1 ? 1 : d; }
-
-namespace {
 template <class KernOf, class SmemOf>
 Pick cached_pick(int dir, int K, int gpad, int n0, int n1, int n2, KernOf kern_of, SmemOf smem_of, int gc)
 {
@@ -766,7 +754,7 @@ Pick cached_pick(int dir, int K, int gpad, int n0, int n1, int n2, KernOf kern_o
         const PickKey &q = g_picks[i].k;
         if (q.dir == dir && q.K == K && q.gpad == gpad && q.n0 == n0 && q.n1 == n1 && q.n2 == n2 && q.cap == key.cap && q.dev == dev) return g_picks[i].p;
     }
-    const Pick p = pick_ng(kern_of, smem_of, gc, g_ng_forced);
+    const Pick p = pick_ng(kern_of, smem_of, gc);
     if (g_npicks < 128) g_picks[g_npicks++] = PickEnt{key, p};
     return p;
 }
@@ -823,9 +811,10 @@ int psg_sa_fused_fwd(const PsgSaFused &f, cudaStream_t st)
                   : f.K == 32 ? cached_pick(0, 32, a.gpad, a.n0, a.n1, a.n2, fwd_kern<32>, smem_of, gc)
                               : cached_pick(0, 16, a.gpad, a.n0, a.n1, a.n2, fwd_kern<16>, smem_of, gc);
     if (pk.ng < 1 || pk.occ < 1 || num_sms() < 1) return PSG_EUNSUPPORTED;
-    // compacted rows: only the device knows the tile count; the persistent CTAs stride over whatever there is
-    const int tiles_for_grid = cp ? (a.ntiles + g_grid_div - 1) / g_grid_div : a.ntiles;
-    const int want = (tiles_for_grid + pk.ng - 1) / pk.ng, cap = num_sms() * pk.occ;
+    // compacted rows: only the device knows the tile count; the persistent CTAs stride over whatever there is.  The grid
+    // is sized for the padded tiles (CTAs without a tile leave after the prologue): a grid for an S3DIS-density guess of
+    // rows / 3 left SA2 (rows / 2, not / 3.6) on 86 of 148 SMs for two rounds of tiles
+    const int want = (a.ntiles + pk.ng - 1) / pk.ng, cap = num_sms() * pk.occ;
     const int grid = want < cap ? want : cap;
     auto kern = x3 ? fwd_kern_cp_x3(pk.ng) : cp ? fwd_kern_cp(pk.ng) : f.K == 32 ? fwd_kern<32>(pk.ng) : fwd_kern<16>(pk.ng);
     { cudaError_t e__ = psg_launch_pdl(kern, dim3(grid), dim3(pk.ng * 160), smem_of(pk.ng), st, 1, a);
@@ -858,8 +847,7 @@ int psg_sa_fused_bwd(const PsgSaFused &f, TView dout, TView dG, int gcols, float
                   : f.K == 32 ? cached_pick(1, 32, a.gpad, a.n0, a.n1, a.n2, bwd_kern<32>, smem_of, gc)
                               : cached_pick(1, 16, a.gpad, a.n0, a.n1, a.n2, bwd_kern<16>, smem_of, gc);
     if (pk.ng < 1 || pk.occ < 1 || num_sms() < 1) return PSG_EUNSUPPORTED;
-    const int tiles_for_grid = cp ? (a.ntiles + g_grid_div - 1) / g_grid_div : a.ntiles;
-    const int want = (tiles_for_grid + pk.ng - 1) / pk.ng, cap = num_sms() * pk.occ;
+    const int want = (a.ntiles + pk.ng - 1) / pk.ng, cap = num_sms() * pk.occ;
     const int grid = want < cap ? want : cap;
     auto kern = x3 ? bwd_kern_cp_x3(pk.ng) : cp ? bwd_kern_cp(pk.ng) : f.K == 32 ? bwd_kern<32>(pk.ng) : bwd_kern<16>(pk.ng);
     { cudaError_t e__ = psg_launch_pdl(kern, dim3(grid), dim3(pk.ng * 160), smem_of(pk.ng), st, 1, a);

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """A/B of library options on BASELINE config 3 (MSG NB, B = 64 x 4096, 10 iterations): time per attack per option setting.
-  python tools/ab_msg.py fp_slabs=0 fp_slabs=1"""
+  python tools/ab_msg.py sa_compact=1 sa_compact=0"""
 import ctypes as C, json, os, sys
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -15,7 +15,7 @@ B = int(os.environ.get("AB_BLOCKS", "64"))
 x = syn.make_blocks(B, 4096, 0).cuda(); torch.manual_seed(5); lab = m(x)[0].argmax(2).cpu().numpy().astype(np.float64)
 atk = torchattacks.NB_attack(m, eps=0.1, alpha=0.05, iters=10)
 ref = None
-for setting in sys.argv[1:] or ["deep=0"]:
+for setting in sys.argv[1:] or ["sa_compact=1", "sa_compact=0"]:
     for kv in setting.split(","):
         k, v = kv.split("="); assert L.psg_set_option(k.encode(), int(v)) == 0, k
     torch.manual_seed(0); out = atk(x, lab); torch.cuda.synchronize()

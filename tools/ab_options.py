@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """A/B of library options at the bench configuration (config[1]: SSG tar-NB, B=16 x 4096, K steps): median attack time
 over repeats (CUDA events, L2 flushed) and the per-family times, per option setting.
-  python tools/ab_options.py deep=0 deep=1 deep=3 deep=3,sa_grid_div=3"""
+  python tools/ab_options.py sa_compact=1 sa_compact=0 fps_cluster=0,nn_grid=1"""
 import ctypes as C, json, os, sys
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -11,7 +11,7 @@ from pointsecguard_b200.engine import MLP_TF32
 from pointsecguard_b200.models.pointnet2_sem_seg import get_model
 
 K = int(os.environ.get("AB_STEPS", "50"))
-DEFAULTS = {"deep": 0, "sa_grid_div": 1, "segsum_warp": 0, "segsum_fast": 1}
+DEFAULTS = {"nn_grid": 0, "fps_cluster": 1, "sa_compact": 1, "x3_fused": 3}
 m = get_model(13); m.load_state_dict(syn.make_state_dict("ssg", init="he")); m = m.cuda().eval(); m.set_mlp_mode(int(os.environ.get("AB_MODE", MLP_TF32)))
 x, labels, mask = bench.make_inputs(16, 0)
 lab = labels.numpy().astype(np.float64)
@@ -19,7 +19,7 @@ xd = x.cuda()
 flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
 atk = torchattacks.tar_NB_attack(m, eps=0.5, alpha=0.1, iters=K, target=7, mask=mask)
 ref = None
-for setting in sys.argv[1:] or ["deep=3"]:
+for setting in sys.argv[1:] or ["sa_compact=1", "sa_compact=0"]:
     opts = dict(DEFAULTS)
     opts.update({k: int(v) for k, v in (kv.split("=") for kv in setting.split(","))})
     for k, v in opts.items():

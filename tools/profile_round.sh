@@ -9,7 +9,6 @@ python tools/primitives_roofline.py --out gpurun_out/pr_primitives_roofline.json
 python tools/family_times.py > gpurun_out/pr_family_times.txt 2>&1
 python tools/attack_overhead.py > gpurun_out/pr_attack_overhead.txt 2>&1
 python tools/l2_stream_bench.py > gpurun_out/pr_l2_stream.json 2> gpurun_out/pr_l2_stream.err
-python tools/deep_trace.py deep=1 > gpurun_out/pr_deep_trace.txt 2>&1
 python tools/gemm_precision.py > gpurun_out/pr_gemm_precision.txt 2>&1
 python tools/determinism_check.py > gpurun_out/pr_determinism.txt 2>&1
 python tools/mode_fuzz.py > gpurun_out/pr_mode_fuzz.txt 2>&1
