@@ -102,7 +102,10 @@ __global__ void __launch_bounds__(kThreads) gemm_tc_kernel(PsgGemmArgs g, int bn
                     tc::bulk_g2s(sB + s * kBBytes + (lane <= kBlk ? 0 : kBHalf) + j * BN * 16, w + ((size_t)(kglob + c + j) * g.Nw + n0) * 4,
                                  (uint32_t)(BN * 16), full);
                 }
-            } else if (use_map && BN == bn_tile) {
+            } else if (use_map && BN == bn_tile && n == kBlk) {
+                // the box is always kBlk planes: a short stage (a source whose width is not a whole number of stages,
+                // e.g. 20 + 12 planes) would deliver more bytes than its expect_tx and never complete; it takes the
+                // per-plane copies below
                 if (lane == 1) psg_tmap_load(sB + s * kBBytes, &wmap, n0, kglob + c, full);
             } else if (lane >= 1 && lane <= n) {
                 const int j = lane - 1;
