@@ -158,8 +158,11 @@ int psg_adam_step(float *param, const float *grad, float *exp_avg, float *exp_av
                   float beta2, float eps, float weight_decay, int step, psg_stream_t stream);
 
 /* ---- dense kNN graph in feature space (SURVEY.md 8f rank 4; ResGCN/gcn_lib/dense/torch_edge.py:32-59) ----
- * x [B,N,C] row-major, C <= 64, k <= 32: nn_idx [B,N,k] (int64, nearest first, the point itself included) = the indices
- * torch.topk(-pairwise_distance(x), k) returns; nn_d2 (optional) the squared distances.  No [B,N,N] matrix is formed. */
+ * x [B,N,C] row-major, any C >= 1, 1 <= k <= min(N, 1024) (else PSG_EINVAL): nn_idx [B,N,k] (int64, nearest first, the
+ * point itself included) = the indices torch.topk(-pairwise_distance(x), k) returns; nn_d2 (optional) the squared distances,
+ * equal bit for bit to psg_pairwise_distance.  Strict (distance, index) order: exact ties by ascending index, NaN distances
+ * after +inf (torch.topk ranks NaN first), so every index lies in [0, N) and appears once per row, also for NaN / inf
+ * features; the top-k of one k is a prefix of the top-k of a larger k.  No workspace, no [B,N,N] matrix is formed. */
 int psg_dense_knn(const float *x, int B, int N, int C, int k, int64_t *nn_idx, float *nn_d2, psg_stream_t stream);
 /* pairwise_distance(x) of torch_edge.py:32-43 as the full [B,N,N] matrix (API completeness, small clouds) */
 int psg_pairwise_distance(const float *x, int B, int N, int C, float *out, psg_stream_t stream);

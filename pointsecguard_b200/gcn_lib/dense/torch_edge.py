@@ -1,11 +1,13 @@
 """Dense dilated kNN graph -- drop-in for ResGCN/gcn_lib/dense/torch_edge.py:6-81 (SURVEY.md section 8f rank 4).
 
 ``dense_knn_matrix`` is the hot op of ResGCN's dynamic graph (one call per block of the network): the reference builds the
-full [B, N, N] distance matrix and runs ``torch.topk`` over it; here ``psg_dense_knn`` (csrc/knn.cu) keeps 128 queries per
-CTA in registers with a sorted top-k list each and streams the cloud through shared memory, so no distance reaches HBM.
+full [B, N, N] distance matrix and runs ``torch.topk`` over it; here ``psg_dense_knn`` (csrc/knn.cu) streams the cloud
+through shared memory and keeps each query's best k on chip, so no distance reaches HBM.  Any feature width C and any
+k * dilation up to min(N, 1024) neighbours: every dilated graph of ResGCN-28 (k * dilation = 16 ... 432).
 Same names, signatures and tensor conventions (x [B, C, N, 1] -> edge_index [2, B, N, k]); CUDA tensors only, no CPU
-fallback.  Limits of the kernel: C <= 64 features, k * dilation <= 32 neighbours.  The sparse ``DilatedKnnGraph``
-(torch_cluster) and the ResGCN model / its colour attacks are outside this repository's scope.
+fallback.  Order: nearest first, exact ties by ascending index; NaN distances (NaN or infinite features) come after +inf,
+whereas ``torch.topk`` ranks NaN first -- so every index is in [0, N) and appears once per row.  The sparse
+``DilatedKnnGraph`` (torch_cluster) and the ResGCN model / its colour attacks are outside this repository's scope.
 """
 from __future__ import annotations
 
@@ -14,6 +16,7 @@ from torch import nn
 
 from ... import _lib as L
 
+MAX_K = 1024          # the most neighbours psg_dense_knn returns per point
 
 def _stream():
     return torch.cuda.current_stream().cuda_stream
@@ -56,12 +59,15 @@ def pairwise_distance(x):
 
 @L.on_device_of
 def dense_knn_matrix(x, k=16):
-    """torch_edge.py:45-59: x [B, C, N, 1] -> stack((nn_idx, center_idx)) [2, B, N, k] (long)."""
+    """torch_edge.py:45-59: x [B, C, N, 1] -> stack((nn_idx, center_idx)) [2, B, N, k] (long); 1 <= k <= min(N, 1024)."""
     if not x.is_cuda:
         raise RuntimeError("pointsecguard_b200.gcn_lib runs on CUDA tensors only; there is no CPU fallback")
     with torch.no_grad():
         xc = x.detach().transpose(2, 1).squeeze(-1).float().contiguous()          # [B, N, C]
         B, N, C = xc.shape
+        if not 1 <= k <= min(N, MAX_K):
+            raise ValueError(f"dense_knn_matrix: k = {k} neighbours requested, but k must lie in [1, min(N, {MAX_K})] "
+                             f"with N = {N} points")
         nn_idx = torch.empty(B, N, k, dtype=torch.int64, device=x.device)
         L.psg_dense_knn(xc.data_ptr(), B, N, C, int(k), nn_idx.data_ptr(), None, _stream())
         center_idx = torch.arange(0, N, device=x.device).repeat(B, k, 1).transpose(2, 1)
