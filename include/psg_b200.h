@@ -120,25 +120,31 @@ int psg_mlp_backward(const psg_mlp *m, const float *dy_base, int dy_wchunks, int
  * points add what training needs.  All reductions are deterministic (fixed partitions, ordered combination). */
 /* nn.BatchNorm{1,2}d.train() + optional ReLU over the rows of z (pointnet_util.py:200-203, :317-319): batch mean /
  * biased variance -> y = relu?((z - mean) * invstd * gamma + beta); running_mean / running_var (may be null) updated in
- * place with `momentum` (variance unbiased); save_mean / save_invstd [C] feed the backward.  C % 4 == 0. */
+ * place with `momentum` (variance unbiased); save_mean / save_invstd [C] feed the backward.  C % 4 == 0, and every view
+ * holds the C columns: 4 * z_wchunks >= C and 4 * y_wchunks >= C (else PSG_EINVAL). */
 size_t psg_bn_workspace(int C);
 int psg_bn_train_forward(const float *z_base, int z_wchunks, int64_t rows, int C, const float *gamma, const float *beta,
                          float *running_mean, float *running_var, float momentum, float eps, float *y_base,
                          int y_wchunks, int relu, float *save_mean, float *save_invstd, void *workspace,
                          size_t workspace_bytes, psg_stream_t stream);
 /* autograd of the same: g = dy * [y > 0] (y_base null: no ReLU); dgamma = sum g xhat, dbeta = sum g,
- * dz = (g - dbeta/n - xhat dgamma/n) gamma invstd (dz may alias dy; rows past the end are zeroed) */
+ * dz = (g - dbeta/n - xhat dgamma/n) gamma invstd (dz may alias dy; rows past the end are zeroed).  4 * wchunks >= C for
+ * dy, z, dz and (when given) y. */
 int psg_bn_train_backward(const float *dy_base, int dy_wchunks, const float *y_base, int y_wchunks, const float *z_base,
                           int z_wchunks, int64_t rows, int C, const float *gamma, const float *save_mean,
                           const float *save_invstd, float *dgamma, float *dbeta, float *dz_base, int dz_wchunks,
                           void *workspace, size_t workspace_bytes, psg_stream_t stream);
 /* weight / bias gradient of a 1x1 conv: dW[cout][k1+k2] (row-major) = dz^T [A1 | A2], db[cout] = column sums of dz
- * (db may be null; accumulate != 0 adds to dW).  Split-K over rows, partial tiles summed in order. */
+ * (db may be null and is overwritten; accumulate != 0 adds to dW).  Split-K over rows, partial tiles summed in order.
+ * Widths: 4 * dz_wchunks >= cout; a1_c0 + ceil(k1 / 4) <= a1_wchunks, and the same for A2 when k2 > 0; k1 % 4 == 0 when
+ * k2 > 0 (else PSG_EINVAL). */
 size_t psg_wgrad_workspace(int cout, int cin, int64_t rows);
 int psg_conv_wgrad(const float *dz_base, int dz_wchunks, int cout, const float *a1_base, int a1_wchunks, int a1_c0, int k1,
                    const float *a2_base, int a2_wchunks, int a2_c0, int k2, int64_t rows, float *dW, float *db,
                    int accumulate, void *workspace, size_t workspace_bytes, psg_stream_t stream);
-/* F.log_softmax over the class logits (pointnet2_sem_seg.py:38) -> logp [rows][ncls] row-major, and its autograd */
+/* F.log_softmax over the class logits (pointnet2_sem_seg.py:38) -> logp [rows][ncls] row-major, and its autograd.
+ * 2 <= ncls <= 16 and 4 * z_wchunks >= ncls; the autograd writes all 16 columns of dz (zeros past ncls), so
+ * dz_wchunks >= 4 (else PSG_EINVAL). */
 int psg_log_softmax_rows(const float *z_base, int z_wchunks, int64_t rows, int ncls, float *logp, psg_stream_t stream);
 int psg_dlogits_from_dlogp(const float *z_base, int z_wchunks, const float *dlogp, int64_t rows, int ncls, float *dz_base,
                            int dz_wchunks, psg_stream_t stream);
@@ -149,7 +155,8 @@ int psg_nll_loss(const float *logp, const int64_t *labels, const float *weight, 
                  float *wsum, void *workspace, size_t workspace_bytes, psg_stream_t stream);
 int psg_nll_loss_backward(const int64_t *labels, const float *weight, int64_t rows, int ncls, const float *grad_out,
                           const float *wsum, float *dlogp, psg_stream_t stream);
-/* x *= m * scale, both T-layout [rows][C] (nn.Dropout(0.5) forward and backward with a 0/1 keep mask, scale 2) */
+/* x *= m * scale, both T-layout [rows][C] (nn.Dropout(0.5) forward and backward with a 0/1 keep mask, scale 2);
+ * 4 * x_wchunks >= C and 4 * m_wchunks >= C */
 int psg_tl_mul(float *x_base, int x_wchunks, const float *m_base, int m_wchunks, int64_t rows, int C, float scale,
                psg_stream_t stream);
 /* torch.optim.Adam step over one flat buffer (train_semseg.py:125-132: betas (0.9, 0.999), eps 1e-8, L2 weight_decay

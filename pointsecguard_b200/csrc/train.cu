@@ -416,6 +416,7 @@ extern "C" int psg_bn_train_forward(const float *z_base, int z_wchunks, int64_t 
                                     void *workspace, size_t workspace_bytes, psg_stream_t stream)
 {
     if (!z_base || !y_base || !gamma || !beta || !save_mean || !save_invstd || !workspace || rows <= 0 || C <= 0 || C % 4) return PSG_EINVAL;
+    if (4 * z_wchunks < C || 4 * y_wchunks < C) return PSG_EINVAL;
     if (workspace_bytes < psg_bn_workspace(C)) return PSG_EWORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
     const int chunks = C / 4;
@@ -445,6 +446,7 @@ extern "C" int psg_bn_train_backward(const float *dy_base, int dy_wchunks, const
     if (!dy_base || !z_base || !gamma || !save_mean || !save_invstd || !dgamma || !dbeta || !dz_base || !workspace || rows <= 0 ||
         C <= 0 || C % 4)
         return PSG_EINVAL;
+    if (4 * dy_wchunks < C || 4 * z_wchunks < C || 4 * dz_wchunks < C || (y_base && 4 * y_wchunks < C)) return PSG_EINVAL;
     if (workspace_bytes < psg_bn_workspace(C)) return PSG_EWORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
     const int chunks = C / 4;
@@ -484,6 +486,10 @@ extern "C" int psg_conv_wgrad(const float *dz_base, int dz_wchunks, int cout, co
 {
     if (!dz_base || !a1_base || !dW || !workspace || cout <= 0 || k1 <= 0 || k2 < 0 || rows <= 0) return PSG_EINVAL;
     if (k2 > 0 && (!a2_base || k1 % 4)) return PSG_EINVAL;
+    // every view must hold the columns it is read for: dz the cout columns of dW / db, A1 (A2) k1 (k2) columns from a1_c0
+    // (a2_c0) on -- a narrower view would read into the next row tile
+    if (4 * dz_wchunks < cout || a1_c0 < 0 || a1_c0 + (k1 + 3) / 4 > a1_wchunks) return PSG_EINVAL;
+    if (k2 > 0 && (a2_c0 < 0 || a2_c0 + (k2 + 3) / 4 > a2_wchunks)) return PSG_EINVAL;
     if (workspace_bytes < psg_wgrad_workspace(cout, k1 + k2, rows)) return PSG_EWORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
     const int cin = k1 + k2;
@@ -507,7 +513,7 @@ extern "C" int psg_conv_wgrad(const float *dz_base, int dz_wchunks, int cout, co
     wgrad_reduce_kernel<<<(total + 255) / 256, 256, 0, st>>>((const float *)workspace, splits, p.npad, p.kpad, cout, cin, dW, accumulate);
     PSG_LAUNCH_CHECK();
     if (db) {
-        const int C = dz_wchunks * 4 < round_up(cout, 4) ? dz_wchunks * 4 : round_up(cout, 4);
+        const int C = round_up(cout, 4);
         const int chunks = C / 4;
         Splits sp = plan_splits(rows, chunks);
         double *part = (double *)((char *)workspace + (((size_t)splits * p.npad * p.kpad * sizeof(float) + 1023) & ~(size_t)1023));
@@ -524,14 +530,16 @@ extern "C" int psg_conv_wgrad(const float *dz_base, int dz_wchunks, int cout, co
 
 extern "C" int psg_log_softmax_rows(const float *z_base, int z_wchunks, int64_t rows, int ncls, float *logp, psg_stream_t stream)
 {
-    if (!z_base || !logp || rows <= 0 || ncls < 2 || ncls > 16) return PSG_EINVAL;
+    if (!z_base || !logp || rows <= 0 || ncls < 2 || ncls > 16 || 4 * z_wchunks < ncls) return PSG_EINVAL;
     return psg_head_logsoftmax(mkv(z_base, z_wchunks, 0), rows, ncls, logp, (cudaStream_t)stream);
 }
 
 extern "C" int psg_dlogits_from_dlogp(const float *z_base, int z_wchunks, const float *dlogp, int64_t rows, int ncls,
                                       float *dz_base, int dz_wchunks, psg_stream_t stream)
 {
-    if (!z_base || !dlogp || !dz_base || rows <= 0 || ncls < 2 || ncls > 16) return PSG_EINVAL;
+    // dz: all 16 columns of the row are written (zeros past ncls)
+    if (!z_base || !dlogp || !dz_base || rows <= 0 || ncls < 2 || ncls > 16 || 4 * z_wchunks < ncls || dz_wchunks < 4)
+        return PSG_EINVAL;
     return psg_dz_from_dlogp(mkv(z_base, z_wchunks, 0), dlogp, rows, ncls, mkv(dz_base, dz_wchunks, 0), (cudaStream_t)stream);
 }
 
@@ -565,7 +573,7 @@ extern "C" int psg_nll_loss_backward(const int64_t *labels, const float *weight,
 extern "C" int psg_tl_mul(float *x_base, int x_wchunks, const float *m_base, int m_wchunks, int64_t rows, int C, float scale,
                           psg_stream_t stream)
 {
-    if (!x_base || !m_base || rows <= 0 || C <= 0 || C % 4) return PSG_EINVAL;
+    if (!x_base || !m_base || rows <= 0 || C <= 0 || C % 4 || 4 * x_wchunks < C || 4 * m_wchunks < C) return PSG_EINVAL;
     cudaStream_t st = (cudaStream_t)stream;
     const long long total = (long long)((rows + 127) / 128) * (C / 4) * 128;
     tl_mul_kernel<<<ew_grid(total), 256, 0, st>>>(mkv(x_base, x_wchunks, 0), mkv(m_base, m_wchunks, 0), rows, C / 4, scale);

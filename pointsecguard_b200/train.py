@@ -141,14 +141,15 @@ class TrainEngine:
         mean = torch.empty(layer.cout, dtype=torch.float32, device=self.dev)
         invstd = torch.empty_like(mean)
         ws = self._bn_workspace(layer.cout)
-        mom = 0.1 if bn.momentum is None else float(bn.momentum)
         track = bn.track_running_stats and bn.running_mean is not None
+        if track:
+            bn.num_batches_tracked += 1
+        # nn.BatchNorm: momentum None is the cumulative average, factor 1 / num_batches_tracked counted after this batch
+        mom = float(bn.momentum) if bn.momentum is not None else (1.0 / float(bn.num_batches_tracked) if track else 0.0)
         L.psg_bn_train_forward(z.ptr, z.wchunks, rows, layer.cout, bn.weight.data_ptr(), bn.bias.data_ptr(),
                                bn.running_mean.data_ptr() if track else None, bn.running_var.data_ptr() if track else None,
                                mom, float(bn.eps), y.ptr, y.wchunks, 1, mean.data_ptr(), invstd.data_ptr(), ws.data_ptr(),
                                ws.numel(), st)
-        if track:
-            bn.num_batches_tracked += 1
         rec.update(y=y, mean=mean, invstd=invstd)
         return rec
 
