@@ -324,9 +324,6 @@ int psg_scene_gather(const double *points, int ld, int label_col, const int32_t 
  * "fps_cluster" (default 1) = cluster FPS kernel for large clouds;
  * "sa_compact" (default 1) = fused set-abstraction branches run on compacted neighbourhood rows (0: padded rows);
  * "x3_fused" (default 3) = 3xTF32 mode: bit 0 fuses the narrow set-abstraction branches, bit 1 fp1 + head;
- * "sm_cap" (default 0 = all) = spread persistent launches over at most that many SMs, so that sub-batches
- * enqueued on different streams share the GPU instead of queueing behind each other;
- * "dbg" (default 0) = debug bits of the tile programs (tools/tile_trace.py);
  * "stream_stages", "stream_stage_bytes", "stream_rings" = ring of psg_debug_l2_stream (measurement only) */
 int psg_set_option(const char *name, int value);
 /* Measurement only (tools/l2_stream_bench.py): `ctas` CTAs each stream `passes` x region_bytes of L2-resident memory into

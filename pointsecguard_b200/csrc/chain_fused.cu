@@ -86,7 +86,6 @@ struct TileArgs {
     const int *labels; float scale, kappa; const float *dlogp;
     float *loss_rows; unsigned char *hit;
     TView zout;
-    int dbg;
     long long *trace;                    // debug: clock64 stamps of CTA 0 ([role][512]; psg_debug_trace), or null
 };
 
@@ -693,7 +692,6 @@ __global__ void __launch_bounds__(NG * 128 + 64, 1) tile_kernel(const __grid_con
 
 int g_sms = 0;
 long long *g_trace = nullptr;
-int g_dbg = 0;
 int g_trace_cap = 0, g_trace_n = 0;
 constexpr size_t kSmemMax = 232448 - 256;      // 227 KB per CTA minus the static barriers
 
@@ -779,11 +777,9 @@ int launch_program(Builder &b, long long rows, cudaStream_t st)
             return PSG_ECUDA;
     }
     a.rows = rows; a.ntiles = (int)((rows + 127) / 128);
-    a.dbg = g_dbg;
     a.trace = psg_tile_trace_slot();
     a.abytes = b.amax_cols * 512;
-    const int sms = (g_psg_sm_cap > 0 && g_psg_sm_cap < g_sms) ? g_psg_sm_cap : g_sms;
-    const int cs = pick_cluster(a, a.ntiles, sms);
+    const int cs = pick_cluster(a, a.ntiles, g_sms);
     a.tcols = (int)pow2cols(b.nmax / cs);
     a.bias_floats = 0;
     for (int o = 0; o < a.nops; ++o) {
@@ -812,7 +808,7 @@ int launch_program(Builder &b, long long rows, cudaStream_t st)
                ((scatters || a.rmstage) ? (size_t)ng * 4 * 32 * 20 : 0) + (a.rmstage ? (size_t)ng * 4 * 4096 : 0) + 128;
     };
     // two tiles in flight share every weight stage; with few tiles one tile per CTA spreads them over more SMs
-    int ng = (cs == 1 && a.ntiles > sms && a.tcols * 2 <= 512 && need(2, 16 * 1024) <= kSmemMax) ? 2 : 1;
+    int ng = (cs == 1 && a.ntiles > g_sms && a.tcols * 2 <= 512 && need(2, 16 * 1024) <= kSmemMax) ? 2 : 1;
     if (b.x3) {
         // operand = [A | A_lo]: the residual copy starts at the widest operand's width, one tile in flight, tensor memory only
         if (cs != 1) return PSG_EUNSUPPORTED;
@@ -841,7 +837,7 @@ int launch_program(Builder &b, long long rows, cudaStream_t st)
     int rc;
     if (cs == 1) {
         const int want = (a.ntiles + ng - 1) / ng;
-        const int grid = want < sms ? want : sms;
+        const int grid = want < g_sms ? want : g_sms;
         if (b.x3) rc = launch_tile<1, 1, true, true>(a, grid, smem, st);
         else if (ts) rc = ng == 2 ? launch_tile<2, 1, true>(a, grid, smem, st) : launch_tile<1, 1, true>(a, grid, smem, st);
         else rc = ng == 2 ? launch_tile<2, 1>(a, grid, smem, st) : launch_tile<1, 1>(a, grid, smem, st);
@@ -1030,6 +1026,5 @@ int psg_fp_stream_bwd(const PsgFpStream &f, TView dy_last, TView dcat, float *dc
     return launch_program(b, f.rows, st);
 }
 
-void psg_tile_set_dbg(int v) { g_dbg = v; }
 long long *psg_tile_trace_slot() { return (g_trace && g_trace_n < g_trace_cap) ? g_trace + (size_t)(g_trace_n++) * 2048 : nullptr; }
 void psg_tile_set_trace(long long *buf, int nlaunches) { g_trace = buf; g_trace_cap = nlaunches; g_trace_n = 0; }

@@ -379,7 +379,8 @@ static int launch_fps_cluster(int ppt, const float *xyz, long long cloud_stride,
     return PSG_OK;
 }
 
-// cluster path for 16384 < N <= 65536 (psg_set_option "fps_cluster"; off until verified on the GPU in this round)
+// cluster kernels for 16384 < N <= 65536 (and few problems of 8192 < N <= 16384), on by default; psg_set_option
+// "fps_cluster" 0 selects the single-CTA kernels, the reference tests/test_gpu_primitives.py matches them against bit for bit
 static int g_fps_cluster = 1;
 void psg_fps_use_cluster(int on) { g_fps_cluster = on; }
 

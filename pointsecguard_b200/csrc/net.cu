@@ -22,7 +22,6 @@
 #include "psg_internal.h"
 
 long long g_psg_launch_count = 0;
-int g_psg_sm_cap = 0;
 // FP levels with fewer 128-row tiles than this run per layer: with a third of the SMs or fewer busy, 64 column-split
 // GEMM CTAs with a deep operand ring beat one cluster per tile (B = 16: fp3 as a tile program 1133 steps/s, per
 // layer 1153)
@@ -472,8 +471,6 @@ extern "C" int psg_set_option(const char *name, int value)
     if (!strcmp(name, "stream_stages")) { psg_stream_tune(value, 0, 0); return PSG_OK; }
     if (!strcmp(name, "stream_stage_bytes")) { psg_stream_tune(0, value, 0); return PSG_OK; }
     if (!strcmp(name, "stream_rings")) { psg_stream_tune(0, 0, value); return PSG_OK; }
-    if (!strcmp(name, "dbg")) { psg_tile_set_dbg(value); return PSG_OK; }
-    if (!strcmp(name, "sm_cap")) { g_psg_sm_cap = value > 0 ? value : 0; return PSG_OK; }
     return PSG_EINVAL;
 }
 

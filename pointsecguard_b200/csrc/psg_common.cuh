@@ -45,7 +45,6 @@ static inline long long round_up_ll(long long x, long long m) { return (x + m - 
 static inline size_t tl_bytes(long long rows, int cpad) { return (size_t)round_up_ll(rows, 128) * cpad * sizeof(float); }
 
 extern long long g_psg_launch_count;   // kernels launched by this library (net.cu)
-extern int g_psg_sm_cap;               // > 0: persistent launches spread over at most this many SMs (net.cu)
 
 // Function attributes (the opt-in to > 48 KB of dynamic shared memory) are per device: one flag per kernel, one bit
 // per device ordinal; setting an attribute twice from racing threads is harmless, so an atomic bit mask is enough.

@@ -151,7 +151,6 @@ struct PsgFpStream {
 bool psg_fp_streamable(const PsgFpStream &f, bool forward);
 int psg_fp_stream_fwd(const PsgFpStream &f, cudaStream_t st);
 int psg_fp_stream_bwd(const PsgFpStream &f, TView dy_last, TView dcat, float *dcat_rm, TView dskip, cudaStream_t st);
-void psg_tile_set_dbg(int v);
 long long *psg_tile_trace_slot();   // next [4][512] block of the debug trace buffer, or null
 void psg_tile_set_trace(long long *buf, int nlaunches);
 // geomgrad.cu: gradient w.r.t. coordinates through grouping and interpolation weights

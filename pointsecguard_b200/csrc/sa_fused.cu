@@ -691,7 +691,7 @@ int num_sms()
             cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
             g_num_sms = 0;
     }
-    return (g_psg_sm_cap > 0 && g_psg_sm_cap < g_num_sms) ? g_psg_sm_cap : g_num_sms;
+    return g_num_sms;
 }
 
 template <int K> void (*fwd_kern(int ng))(SaFwdArgs)
@@ -738,7 +738,7 @@ Pick pick_ng(KernOf kern_of, SmemOf smem_of, int gc)
     return best;
 }
 
-struct PickKey { int dir, K, gpad, n0, n1, n2, cap, dev; };
+struct PickKey { int dir, K, gpad, n0, n1, n2, dev; };
 struct PickEnt { PickKey k; Pick p; };
 PickEnt g_picks[128];
 int g_npicks = 0;
@@ -749,10 +749,10 @@ Pick cached_pick(int dir, int K, int gpad, int n0, int n1, int n2, KernOf kern_o
     // the pick also carries a side effect of ctas_per_sm (the per-device shared-memory opt-in), so it is keyed by device
     int dev = 0;
     cudaGetDevice(&dev);
-    const PickKey key{dir, K, gpad, n0, n1, n2, g_psg_sm_cap, dev};
+    const PickKey key{dir, K, gpad, n0, n1, n2, dev};
     for (int i = 0; i < g_npicks; ++i) {
         const PickKey &q = g_picks[i].k;
-        if (q.dir == dir && q.K == K && q.gpad == gpad && q.n0 == n0 && q.n1 == n1 && q.n2 == n2 && q.cap == key.cap && q.dev == dev) return g_picks[i].p;
+        if (q.dir == dir && q.K == K && q.gpad == gpad && q.n0 == n0 && q.n1 == n1 && q.n2 == n2 && q.dev == dev) return g_picks[i].p;
     }
     const Pick p = pick_ng(kern_of, smem_of, gc);
     if (g_npicks < 128) g_picks[g_npicks++] = PickEnt{key, p};

@@ -156,7 +156,7 @@ class Engine:
         return bool((head == 0xA5).all().item()) and bool((tail == 0xA5).all().item())
 
     def _stream(self):
-        """Stream the C library enqueues on: the one set with ``use_stream`` (sub-batch pipelining,
+        """Stream the C library enqueues on: the one set with ``use_stream`` (the geometry head start's tail engine,
         torchattacks/attacks/nontarget.py) or torch's current stream."""
         return self._stream_handle if self._stream_handle is not None else torch.cuda.current_stream(self.device).cuda_stream
 

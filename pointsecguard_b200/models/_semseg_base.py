@@ -51,23 +51,18 @@ class SemSegBase(nn.Module):
     """get_model.forward of pointnet2_sem_seg.py:22-40 / pointnet2_sem_seg_msg.py:23-41."""
 
     arch = "ssg"
-    # default MLP mode of the eval-mode (attack) engine; PSG_DEFAULT_MLP overrides it process-wide (A/B of the defaults)
-    mlp_mode = int(__import__("os").environ.get("PSG_DEFAULT_MLP", MLP_FP32))
+    # default MLP mode of the eval-mode (attack) engine (set_mlp_mode changes it per model)
+    mlp_mode = MLP_FP32
     # autograd of forward(): False = gradient through the features only (all the colour attacks need);
     # True = also through the geometry (centred neighbour coordinates, interpolation weights), which
     # is what the reference's autograd produces on input channels 0:3
     xyz_grad = False
-
-    # number of independent sub-batches an attack pipelines over CUDA streams ("auto": by batch size)
-    sub_batches = "auto"
 
     def _init_runtime(self):
         self._engine = None
         self._engine_key = None
         self._generation = 0
         self._shard = None
-        self._sub_engines = []
-        self._sub_streams = []
 
     def set_shard(self, shard):
         """Multi-GPU runs: declare that the batches this replica sees are ``shard``
@@ -94,26 +89,7 @@ class SemSegBase(nn.Module):
             self._engine = Engine(self.describe(), device, self.mlp_mode)
             self._engine_key = key
             self._engine.set_shard(self._shard)
-            self._sub_engines = []
         return self._engine
-
-    def sub_engines(self, device, count: int, primary=None):
-        """``count`` engines (same folded weights, own workspace) with one CUDA stream each.  The
-        attacks split a batch into independent sub-batches and enqueue them round-robin: the deep
-        levels of the network are latency-bound chains of small launches, and blocks are independent
-        in every op of the path, so sub-batches overlap on the GPU."""
-        if primary is None:                     # (the parameter walk of engine() costs ~0.5 ms: callers that just made it pass it in)
-            primary = self.engine(device)
-        if count <= 1:
-            return [primary], [None]
-        while len(self._sub_engines) < count - 1:
-            self._sub_engines.append(Engine(self.describe(), primary.device, self.mlp_mode))
-        while len(self._sub_streams) < count:
-            self._sub_streams.append(torch.cuda.Stream(primary.device))
-        engs = [primary] + self._sub_engines[: count - 1]
-        for e in engs:
-            e.set_mlp_mode(self.mlp_mode)
-        return engs, self._sub_streams[:count]
 
     def tail_engine(self, device, primary=None):
         """A second engine (same folded weights, own workspace) and a side stream: the norm-bounded attacks compute the
@@ -131,8 +107,6 @@ class SemSegBase(nn.Module):
         self.mlp_mode = mode
         if self._engine is not None:
             self._engine.set_mlp_mode(mode)
-            for e in self._sub_engines:
-                e.set_mlp_mode(mode)
             if getattr(self, "_tail", None) is not None:
                 self._tail.set_mlp_mode(mode)
             self._engine_key = self._param_key(self._engine.device)

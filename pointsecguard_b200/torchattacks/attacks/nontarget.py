@@ -25,137 +25,85 @@ class NB_attack(Attack):
         return _nb_loop(self, images, labels, target=-1, mask=None)
 
 
-def _sub_batches(model, B):
-    import os
-    want = os.environ.get("PSG_SUBBATCH") or getattr(model, "sub_batches", "auto")
-    if want == "auto":
-        # measured on B200 at B=16: the persistent fused kernels already fill the SMs, sub-batch overlap
-        # gains nothing there (65.5 ms / 50 steps with 1 or 4 sub-batches); kept as an opt-in knob
-        want = 1
-    return max(1, min(int(want), B))
-
-
 def _head_start(model, t):
     """Forwards of a geometry chunk that run on the primary engine while the rest of the chunk's geometry is computed
-    on a side stream (0 = no pipelining).  ``model.geometry_head`` / PSG_GEOHEAD override the default of 4 (measured at B = 16: 20 iterations 14.55 -> 14.14 ms, 50 iterations 34.0 -> 33.75 ms)."""
-    import os
-    want = os.environ.get("PSG_GEOHEAD")
-    want = int(want) if want is not None else int(getattr(model, "geometry_head", 4))
+    on a side stream (0 = no pipelining).  ``model.geometry_head`` overrides the default of 4 (measured at B = 16: 20 iterations 14.55 -> 14.14 ms, 50 iterations 34.0 -> 33.75 ms)."""
+    want = int(getattr(model, "geometry_head", 4))
     if want <= 0 or t < 4 * want:
         return 0
     return want
 
 
 def _nb_loop(atk, images, labels, target, mask):
-    from pointsecguard_b200 import distributed as D
     eng = atk._engine(images)
     dev = images.device
     B, C, N = images.shape
     src = images.detach()
     # nontarget.py:34: sum-CE / N;  target.py:38: mean CE over the B*N points
     scale = 1.0 / N if target < 0 else 1.0 / (B * N)
-    # Blocks are independent in every op of the path: split the batch into sub-batches, one engine and
-    # one CUDA stream each, and enqueue their steps round-robin so the latency-bound deep levels of
-    # one sub-batch overlap the others.  FPS starts are drawn ONCE for the whole batch (the
-    # reference's draw, pointnet_util.py:75) and sliced.
-    nsub = _sub_batches(atk.model, B)
-    engs, streams = atk.model.sub_engines(dev, nsub, primary=eng)
-    if nsub > 1:
-        # each sub-batch's persistent kernels take an equal share of the SMs, so the streams really overlap
-        from pointsecguard_b200 import _lib as L
-        sms = torch.cuda.get_device_properties(dev).multi_processor_count
-        L.psg_set_option(b"sm_cap", max(1, sms // nsub))
-    whole = eng.shard if eng.shard is not None else D.Shard(B, 0, B)
-    parts = [D.shard_for(B, i, nsub) for i in range(nsub)]
     chunk = max(1, min(atk.iters, _MAX_PROBLEMS // B))
     cur = torch.cuda.current_stream()
-    fork = torch.cuda.Event()
-    fork.record(cur)
-    for e, st_, p in zip(engs, streams, parts):
-        e.use_stream(st_)
-        if st_ is not None:
-            st_.wait_event(fork)
-        e.bind(p.size, N, chunk)
-        e.set_xyz_grad(False)                       # colour attack: no geometric gradient (decided before the geometry pass)
-        e.set_input(p.slice(src))
-    sizes = [N] + eng.npoints[:3]
+    eng.use_stream(None)                            # on `cur`: the head start's events order the tail engine against it
+    eng.bind(B, N, chunk)
+    eng.set_xyz_grad(False)                         # colour attack: no geometric gradient (decided before the geometry pass)
+    eng.set_input(src)
     adv = ori = lab = msk = None
-    try:
-        done = 0
-        while done < atk.iters:
-            t = min(chunk, atk.iters - done)
-            starts = D.draw_starts(sizes, t, whole)                       # int32 [4, t, B]
-            # Head start (single sub-batch): the geometry pass is a latency chain (1360 dependent FPS rounds) whatever the
-            # number of forwards, so the first `head` forwards get their own small pass on the primary engine and the loop
-            # starts on them, while a second engine (own workspace, side stream) computes the geometry of the remaining
-            # forwards beside those first steps.  Same draws, same kernels, same values: results are bit-identical.
-            head = _head_start(atk.model, t) if nsub == 1 else 0
-            tail = tail_ready = None
-            if head:
-                tail, side = atk.model.tail_engine(dev, eng)
-                tail.bind(B, N, t - head)
-                tail.set_xyz_grad(False)
-                fork2 = torch.cuda.Event()
-                fork2.record(cur)
-                side.wait_event(fork2)
-                tail.use_stream(side)
-                try:
-                    tail.set_input(src)
-                    tail.geometry(starts[:, head:].contiguous())
-                    tail_ready = torch.cuda.Event()
-                    tail_ready.record(side)
-                finally:
-                    tail.use_stream(None)
-                eng.geometry(starts[:, :head].contiguous())
-            else:
-                for e, p in zip(engs, parts):
-                    e.geometry(p.slice(starts.permute(2, 0, 1)).permute(1, 2, 0).contiguous())
-            if adv is None:
-                # the loop's own tensors are made AFTER the first geometry pass is enqueued: their host work (label / mask
-                # conversion and upload, clones) then runs while the GPU computes FPS / ball query / 3-NN instead of before it
-                adv = images.detach().clone(memory_format=torch.contiguous_format)
-                ori = images.detach()[:, 3:6].contiguous()
-                lab = atk._labels_i32(labels, dev) if target < 0 else None
-                msk = atk._mask_u8(mask, B, N, dev) if mask is not None else None
-                if msk is not None and B > 1 and getattr(mask, "ndim", 2) == 1:
-                    # target.py:26,36 with a batch: the cost reads outputs[0] only, so the gradient of every other block is
-                    # zero and sign(0) = 0 leaves it where it is -- the reference attacks block 0 alone.  A [B,N] mask
-                    # attacks every block.
-                    msk = msk.clone()
-                    msk[1:] = 0
-                if nsub > 1:
-                    # side streams read these tensors: order them after their creation on the current stream
-                    ready = torch.cuda.Event()
-                    ready.record(cur)
-                    for st_ in streams:
-                        if st_ is not None:
-                            st_.wait_event(ready)
-            if head:
-                for i in range(head):
-                    eng.nb_attack(adv, ori, msk, lab, target, 1, i, atk.alpha, atk.eps, scale)
-                cur.wait_event(tail_ready)
-                tail.copy_input_from(eng)          # the PROJECTED colours of the head's last update (adv holds the un-projected ones)
-                for i in range(t - head):
-                    tail.nb_attack(adv, ori, msk, lab, target, 1, i, atk.alpha, atk.eps, scale)
-                if done + t < atk.iters:
-                    eng.copy_input_from(tail)      # the next chunk starts on the primary engine again
-            else:
-                for i in range(t):
-                    for e, p in zip(engs, parts):
-                        e.nb_attack(p.slice(adv), p.slice(ori), p.slice(msk) if msk is not None else None,
-                                    p.slice(lab) if lab is not None else None, target, 1, i, atk.alpha, atk.eps, scale)
-            done += t
-        if adv is None:                                                    # iters == 0
+    done = 0
+    while done < atk.iters:
+        t = min(chunk, atk.iters - done)
+        starts = eng.draw_starts(t)                                     # int32 [4, t, B]
+        # Head start: the geometry pass is a latency chain (1360 dependent FPS rounds) whatever the number of forwards, so
+        # the first `head` forwards get their own small pass on the primary engine and the loop starts on them, while a
+        # second engine (own workspace, side stream) computes the geometry of the remaining forwards beside those first
+        # steps.  Same draws, same kernels, same values: results are bit-identical.
+        head = _head_start(atk.model, t)
+        tail = tail_ready = None
+        if head:
+            tail, side = atk.model.tail_engine(dev, eng)
+            tail.bind(B, N, t - head)
+            tail.set_xyz_grad(False)
+            fork = torch.cuda.Event()
+            fork.record(cur)
+            side.wait_event(fork)
+            tail.use_stream(side)
+            try:
+                tail.set_input(src)
+                tail.geometry(starts[:, head:].contiguous())
+                tail_ready = torch.cuda.Event()
+                tail_ready.record(side)
+            finally:
+                tail.use_stream(None)
+            eng.geometry(starts[:, :head].contiguous())
+        else:
+            eng.geometry(starts)
+        if adv is None:
+            # the loop's own tensors are made AFTER the first geometry pass is enqueued: their host work (label / mask
+            # conversion and upload, clones) then runs while the GPU computes FPS / ball query / 3-NN instead of before it
             adv = images.detach().clone(memory_format=torch.contiguous_format)
-    finally:
-        for e, st_ in zip(engs, streams):
-            if st_ is not None:
-                join = torch.cuda.Event()
-                join.record(st_)
-                cur.wait_event(join)
-            e.use_stream(None)
-        if nsub > 1:
-            L.psg_set_option(b"sm_cap", 0)
+            ori = images.detach()[:, 3:6].contiguous()
+            lab = atk._labels_i32(labels, dev) if target < 0 else None
+            msk = atk._mask_u8(mask, B, N, dev) if mask is not None else None
+            if msk is not None and B > 1 and getattr(mask, "ndim", 2) == 1:
+                # target.py:26,36 with a batch: the cost reads outputs[0] only, so the gradient of every other block is
+                # zero and sign(0) = 0 leaves it where it is -- the reference attacks block 0 alone.  A [B,N] mask
+                # attacks every block.
+                msk = msk.clone()
+                msk[1:] = 0
+        if head:
+            for i in range(head):
+                eng.nb_attack(adv, ori, msk, lab, target, 1, i, atk.alpha, atk.eps, scale)
+            cur.wait_event(tail_ready)
+            tail.copy_input_from(eng)          # the PROJECTED colours of the head's last update (adv holds the un-projected ones)
+            for i in range(t - head):
+                tail.nb_attack(adv, ori, msk, lab, target, 1, i, atk.alpha, atk.eps, scale)
+            if done + t < atk.iters:
+                eng.copy_input_from(tail)      # the next chunk starts on the primary engine again
+        else:
+            for i in range(t):
+                eng.nb_attack(adv, ori, msk, lab, target, 1, i, atk.alpha, atk.eps, scale)
+        done += t
+    if adv is None:                                                        # iters == 0
+        adv = images.detach().clone(memory_format=torch.contiguous_format)
     atk.model._generation += 1
     return adv
 

@@ -404,7 +404,7 @@ def invalidate_eval_caches(model):
     """Parameters / running statistics were (or are about to be) changed through raw pointers: drop the folded eval-mode
     engines built from the old values."""
     if hasattr(model, "_engine"):
-        model._engine, model._engine_key, model._sub_engines = None, None, []
+        model._engine, model._engine_key = None, None
     for m in model.modules():
         m.__dict__.pop("_psg_chains", None)
 

@@ -62,6 +62,9 @@ def test_argument_errors_are_status_codes_not_crashes():
         L.psg_net_forward(None, 0, None, None, None)
     with pytest.raises(L.PsgError):
         L.psg_nu_step(None, None, 0, 0, -1, 10, 0.1, 0.0, 1.0, 0.01, 1.0, 0, 4096.0, 0.07, 0, 0, None, None)
+    # names that are not library switches
+    for name in (b"no_such_option", b"sm_cap", b"dbg"):
+        assert L._cdll.psg_set_option(name, 1) == L.PSG_EINVAL
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU behaviour")

@@ -1,5 +1,5 @@
-"""GPU tests of the API-surface rows that the sem-seg attack path itself never executes (SURVEY.md a6, a11), of the
-1-D-mask batch behaviour of tar_NB_attack, and of the sub-batch pipelining knob."""
+"""GPU tests of the API-surface rows that the sem-seg attack path itself never executes (SURVEY.md a6, a11) and of the
+1-D-mask batch behaviour of tar_NB_attack."""
 import os
 
 import numpy as np
@@ -46,14 +46,11 @@ def test_get_loss_vs_reference(golden_dir, arch):
     np.testing.assert_allclose(pred.grad.cpu().numpy(), g["dpred"], rtol=1e-5, atol=1e-8)
 
 
-def _ssg(mode="fp32"):
-    from pointsecguard_b200.engine import MLP_FP32, MLP_TF32
+def _ssg():
     from pointsecguard_b200.models.pointnet2_sem_seg import get_model
     m = get_model(13)
     m.load_state_dict(syn.load_checkpoint("ssg"))
-    m = m.cuda().eval()
-    m.set_mlp_mode(MLP_TF32 if mode == "tf32" else MLP_FP32)
-    return m
+    return m.cuda().eval()
 
 
 def test_tar_nb_1d_mask_on_a_batch_attacks_block_0_only():
@@ -95,19 +92,3 @@ def test_tar_nb_leaves_unmasked_points_unclamped():
     # the model input of the next forward kept them too: a clean forward of adv equals a forward where they were never clamped
     assert float(adv[0, 3, far].max()) == pytest.approx(1.7)
 
-
-@pytest.mark.parametrize("mode", ["fp32", "tf32"])
-def test_sub_batch_pipelining_is_bit_identical(monkeypatch, mode):
-    """PSG_SUBBATCH > 1 splits the batch over engines pinned to side streams; the result must not change."""
-    from pointsecguard_b200 import torchattacks
-    m = _ssg(mode)
-    x, labels = syn.make_painted_blocks(8, 2048, 9)
-    xd, lab = x.cuda(), labels.numpy().astype(np.float64)
-    outs = []
-    for nsub in ("1", "4", "4", "2"):
-        monkeypatch.setenv("PSG_SUBBATCH", nsub)
-        torch.manual_seed(0)
-        outs.append(torchattacks.NB_attack(m, eps=0.1, alpha=0.05, iters=6)(xd, lab).clone())
-        torch.cuda.synchronize()
-    for o in outs[1:]:
-        assert torch.equal(o, outs[0])

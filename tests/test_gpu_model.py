@@ -233,21 +233,6 @@ def test_sharded_attack_equals_full_batch_attack():
     assert torch.equal(counters, c_full)
 
 
-def test_sub_batch_pipelining_is_exact():
-    """Splitting a batch into sub-batches on separate CUDA streams (model.sub_batches) changes nothing."""
-    from pointsecguard_b200 import torchattacks
-    m = _model("ssg")
-    x = syn.make_blocks(4, 2048, 6).cuda()
-    lab = syn.zband_labels(x.cpu()).numpy().astype(np.float64)
-    outs = []
-    for nsub in (1, 2, 4):
-        m.sub_batches = nsub
-        torch.manual_seed(8)
-        outs.append(torchattacks.NB_attack(m, eps=0.1, alpha=0.05, iters=3)(x, lab))
-    m.sub_batches = "auto"
-    assert torch.equal(outs[0], outs[1]) and torch.equal(outs[0], outs[2])
-
-
 @pytest.mark.parametrize("arch", ["ssg", "msg"])
 def test_coordinate_gradient_vs_reference_golden(golden_dir, arch):
     """With model.xyz_grad the autograd of forward() is complete on all nine channels: channels 0:3 get

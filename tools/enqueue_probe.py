@@ -12,4 +12,4 @@ torch.cuda.synchronize()
 from pointsecguard_b200 import _lib as L
 l0 = L.psg_launch_count()
 t0 = time.perf_counter(); adv = atk(x, ln); t1 = time.perf_counter(); torch.cuda.synchronize(); t2 = time.perf_counter()
-print("nsub", os.environ.get("PSG_SUBBATCH"), "enqueue ms", (t1 - t0) * 1e3, "total ms", (t2 - t0) * 1e3, "launches", L.psg_launch_count() - l0)
+print("enqueue ms", (t1 - t0) * 1e3, "total ms", (t2 - t0) * 1e3, "launches", L.psg_launch_count() - l0)

@@ -20,7 +20,6 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--blocks", type=int, default=16)
     ap.add_argument("--launches", type=int, default=12)
-    ap.add_argument("--dbg", type=int, default=0)
     ap.add_argument("--raw", action="store_true", help="print the raw stamp deltas of every launch (fused SA kernels included)")
     args = ap.parse_args()
     from pointsecguard_b200 import _lib as L
@@ -39,7 +38,6 @@ def main():
     mk(5)(xd, lab)
     torch.cuda.synchronize()
     buf = torch.zeros(args.launches, 4, 512, dtype=torch.int64, device=dev)
-    L.psg_set_option(b"dbg", args.dbg)
     L.psg_debug_trace(buf.data_ptr(), args.launches)
     mk(1)(xd, lab)
     torch.cuda.synchronize()
@@ -72,9 +70,6 @@ def main():
         base = min(x for x in (w0[0], w1[0] if w1[0] else w0[0], mm[0] if mm[0] else w0[0]))
         print(f"--- tile launch {li}: worker0 {n0} stamps, worker1 {int((w1 != 0).sum())}, mma {int((mm != 0).sum())}; "
               f"span {(max(w0.max(), w1.max()) - base) / 1.9e3:.1f} us (cycles / 1.9 GHz)")
-        if args.dbg & 8:
-            n = int((w0 != 0).sum())
-            print("raw w0 deltas", [int(w0[i + 1] - w0[i]) for i in range(n - 1)])
         for name, w in (("w0", w0), ("w1", w1)):
             n = int((w != 0).sum())
             rows = []
