@@ -192,6 +192,11 @@ typedef struct {
     int mlp_mode;               /* 0 = fp32 CUDA-core GEMM (exact), 1 = tcgen05 TF32 (fused kernels), 2 = tcgen05 3xTF32 (per layer, fp32-grade) */
 } psg_net_desc;
 
+/* Networks psg_net_create accepts (it returns NULL for anything else): 3-16 input channels, 2-16 classes; per SA level
+ * 1-2 branches with nsample 16 or 32, npoint >= 3 and 1-3 layers; 1-3 layers per FP level; any hidden width; branch,
+ * FP and conv1 outputs multiples of 16.  psg_net_bind takes any N >= npoint of SA1 (each npoint at most the previous
+ * level's).  Every accepted network runs in every mode: where a width or count rules out a fused kernel or tile
+ * program, that level runs per layer (tests/test_gpu_archs.py). */
 typedef struct psg_net psg_net;
 psg_net *psg_net_create(const psg_net_desc *desc);
 void psg_net_destroy(psg_net *net);

@@ -999,10 +999,19 @@ int psg_fp_stream_fwd(const PsgFpStream &f, cudaStream_t st)
     return launch_program(b, f.rows, st);
 }
 
+// the store epilogue writes its second destination in whole 32-column groups, and only the first op (columns 0..255)
+// carries it
+int psg_fp_stream_skip_cols(const PsgFpStream &f)
+{
+    if (f.C1 % 32) return 0;
+    return f.C1 < 256 ? f.C1 : 256;
+}
+
 // dY_last (pre-activation gradient, already masked) -> dgrad chain -> d[skip | interp] stored to dcat
 int psg_fp_stream_bwd(const PsgFpStream &f, TView dy_last, TView dcat, float *dcat_rm, TView dskip, cudaStream_t st)
 {
     Builder b;
+    const int skip_cols = dskip.base ? psg_fp_stream_skip_cols(f) : 0;
     for (int j = f.nl - 1; j >= 0; --j) {
         const int nin = j > 0 ? f.n[j - 1] : f.C1 + f.C2;
         if (j > 0) {
@@ -1015,7 +1024,7 @@ int psg_fp_stream_bwd(const PsgFpStream &f, TView dy_last, TView dcat, float *dc
                 TileOp *o = b.add(f.wb[0], f.nwb[0], c0, 0, n, f.n[0] / 4, 0);
                 o->epi = EPI_STORE; o->out = dcat; o->out.c0 += c0 / 4;
                 if (dcat_rm) { o->rm = dcat_rm + c0; o->rm_stride = f.C1 + f.C2; }
-                if (dskip.base && c0 == 0 && f.C1 % 32 == 0) { o->out2 = dskip; o->out2_cols = f.C1 < n ? f.C1 : n; }
+                if (c0 == 0 && skip_cols) { o->out2 = dskip; o->out2_cols = skip_cols; }
                 if (f.nl == 1 && c0 == 0) o->pre = PRE_LOAD;
             }
         }

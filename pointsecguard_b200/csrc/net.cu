@@ -973,7 +973,7 @@ extern "C" int psg_net_backward(psg_net *n, int t, float *grad_x, psg_stream_t s
         if (f == 0) { mlps[nl] = n->conv1; Ys[nl] = n->H; ++nl; mlps[nl] = n->conv2; Ys[nl] = n->Z; ++nl; }
         int cat_buf = 0;
         const float *rm_src = nullptr; int rm_stride = 0;      // row-major copy of d[interp] when a fused kernel produced it
-        bool skip_done = false;                                 // d[skip] already written into dfeat[f] by the producing kernel
+        int skip_done = 0;                                      // leading columns of d[skip] the producing kernel already wrote into dfeat[f]
         if (f == 0 && head_fused_now(n)) {
             if (!n->loss.set) return PSG_EINVAL;
             FpLevel &C = n->fp[1];
@@ -988,19 +988,21 @@ extern "C" int psg_net_backward(psg_net *n, int t, float *grad_x, psg_stream_t s
         } else if (f > 0 && n->mode == 1 && F.streamed) {
             PsgFpStream q = fp_stream_desc(n, f, t, TView{nullptr, 0, 0});
             cat_buf = top_buf == 0 ? 1 : 0;
-            // the skip part of the gradient goes straight into dfeat[f] (no copy kernel)
+            // the skip part of the gradient goes straight into dfeat[f] as far as the tile program covers it
             PSG_RUN(PF_FP_BWD, psg_fp_stream_bwd(q, top, tv(n->S[cat_buf], F.C1 + F.C2), n->Srm, tv(n->dfeat[f], n->wfeat[f]), st));
             rm_src = n->Srm + F.C1; rm_stride = F.C1 + F.C2;
-            skip_done = true;
+            skip_done = psg_fp_stream_skip_cols(q);
         } else if (f > 0 && n->mode >= 1 && F.C1) {
             TView dsk = tv(n->dfeat[f], n->wfeat[f]);
             PSG_TRY(chain_bwd(n, mlps, Ys, nl, rows, top, top_buf, &cat_buf, st, &dsk, F.C1));
-            skip_done = true;
+            skip_done = F.C1;
         } else {
             PSG_TRY(chain_bwd(n, mlps, Ys, nl, rows, top, top_buf, &cat_buf, st));
         }
         const int catw = F.C1 + F.C2;
-        if (F.C1 && !skip_done) PSG_RUN(PF_COPY, psg_copy_cols(tv(n->S[cat_buf], catw), tv(n->dfeat[f], n->wfeat[f]), rows, F.C1, 0, st));
+        if (F.C1 > skip_done)
+            PSG_RUN(PF_COPY, psg_copy_cols(tv(n->S[cat_buf], catw, skip_done), tv(n->dfeat[f], n->wfeat[f], skip_done), rows,
+                                           F.C1 - skip_done, 0, st));
         // interpolation backward: scatter the three weighted copies to the coarse level, in CSR order
         const size_t go = (size_t)t * B;
         if (n->xyz_grad) {

@@ -150,7 +150,10 @@ struct PsgFpStream {
 };
 bool psg_fp_streamable(const PsgFpStream &f, bool forward);
 int psg_fp_stream_fwd(const PsgFpStream &f, cudaStream_t st);
+// psg_fp_stream_bwd also writes the first psg_fp_stream_skip_cols(f) columns of d[skip] into dskip; the caller copies
+// the remaining C1 - psg_fp_stream_skip_cols(f) columns out of dcat
 int psg_fp_stream_bwd(const PsgFpStream &f, TView dy_last, TView dcat, float *dcat_rm, TView dskip, cudaStream_t st);
+int psg_fp_stream_skip_cols(const PsgFpStream &f);
 long long *psg_tile_trace_slot();   // next [4][512] block of the debug trace buffer, or null
 void psg_tile_set_trace(long long *buf, int nlaunches);
 // geomgrad.cu: gradient w.r.t. coordinates through grouping and interpolation weights

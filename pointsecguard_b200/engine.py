@@ -68,6 +68,9 @@ class Engine:
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
         self._keep: List[np.ndarray] = []
+        if any(len(sa["mlps"]) > 2 or any(len(m) > 3 for m in sa["mlps"]) for sa in layers["sa"]) or \
+                any(len(m) > 3 for m in layers["fp"]):
+            raise L.PsgError("psg_net_create takes at most 2 branches per SA level and 3 layers per branch and FP level")
         d = L.NetDesc()
         d.in_channels = layers["in_channels"]
         d.num_classes = layers["num_classes"]

@@ -22,8 +22,6 @@ Measured on a B200 (1000 W), worst case over the 12 cases:
     sign agreement        0.9850          0.959                       0.975
 and per case the plain deviation is at least 2.8x (gradient) and 4.5x (logp) the TF32-exact one (asserted: 2x).
 """
-import ctypes as C
-
 import numpy as np
 import pytest
 import torch
@@ -90,26 +88,27 @@ def _cpu_geometry(x, arch):
     from oracle import pointnet2_oracle as PO
     B = x.shape[0]
     xyz = [x[:, :3].permute(0, 2, 1).contiguous()]
-    geom = {"xyz": {}, "ball": {}, "nn_idx": {}, "nn_w": {}}
+    geom = {"xyz": {}, "fps": {}, "ball": {}, "nn_idx": {}, "nn_w": {}, "nn_d2": {}}
     for l, (S, radii, ks) in enumerate(PO._SA[arch], start=1):
         start = torch.randint(0, xyz[-1].shape[1], (B,), dtype=torch.long)
         fps = G.fps(xyz[-1], S, start)
         new = PO.index_points(xyz[-1], fps)
         for b, (r, K) in enumerate(zip(radii, ks)):
             geom["ball"][(l, b)] = G.ball_query(r, K, xyz[-1], new)
-        geom["xyz"][l] = new
+        geom["xyz"][l], geom["fps"][l] = new, fps
         xyz.append(new)
     for f in range(4):
-        idx, _, w = G.three_nn(xyz[f], xyz[f + 1])
-        geom["nn_idx"][f], geom["nn_w"][f] = idx, w
+        idx, d2, w = G.three_nn(xyz[f], xyz[f + 1])
+        geom["nn_idx"][f], geom["nn_w"][f], geom["nn_d2"][f] = idx, w, d2
     return geom
 
 
 @pytest.mark.parametrize("arch", ["ssg", "msg"])
 def test_plain_reference_matches_the_cpu_oracle(arch):
-    """The network walk of tf32_oracle (plain fp64 mode) against the CPU oracle model (unfolded BatchNorm, its own
-    geometry) at B = 1, N = 1024: log-probabilities and input gradient.  The TF32 mode of the same walk differs from
-    both by the TF32 rounding and no more."""
+    """The network walk of tf32_oracle (plain fp64 mode, differentiable in the coordinates) against the CPU oracle
+    model (unfolded BatchNorm, its own geometry, autograd through centres, centred neighbours and inverse-distance
+    weights) at B = 1, N = 1024: log-probabilities and the input gradient on all nine channels.  The TF32 mode of the
+    same walk differs from both by the TF32 rounding and no more."""
     from oracle import pointnet2_oracle as PO
     if arch == "ssg":
         from pointsecguard_b200.models.pointnet2_sem_seg import get_model
@@ -130,20 +129,27 @@ def test_plain_reference_matches_the_cpu_oracle(arch):
     res = {}
     for tf32 in (False, True):
         x = x0.double().requires_grad_(True)
-        z, l4 = TO.forward(desc, geom, x, tf32)
+        z, l4 = TO.forward(desc, geom, x, tf32, xyz_grad=True)
         g = TO.input_gradient(z, x, TO.dz_ce(z, y.view(1, -1), 1.0 / 1024))
         res[tf32] = (torch.log_softmax(z, -1).detach(), g)
-    # channels 0:3 of the oracle's gradient also carry the geometric path; 3:9 reach the loss through features only
-    go = xo.grad[:, 3:]
+    go = xo.grad
     lp, g = res[False]
     err = (lp - lo.detach()).abs().max().item()
-    rel = ((g[:, 3:] - go).norm() / go.norm()).item()
+    rel = ((g - go).norm() / go.norm()).item()
+    rel_xyz = ((g[:, :3] - go[:, :3]).norm() / go[:, :3].norm()).item()
     lp1, g1 = res[True]
     err1 = (lp1 - lo.detach()).abs().max().item()
-    rel1 = ((g1[:, 3:] - go).norm() / go.norm()).item()
-    print(f"{arch}: plain vs oracle logp {err:.2e} grad rel {rel:.2e} | tf32 vs oracle logp {err1:.2e} grad rel {rel1:.2e}")
+    rel1 = ((g1 - go).norm() / go.norm()).item()
+    # without the coordinate terms channels 0:3 carry the feature path only, far from the oracle's
+    x = x0.double().requires_grad_(True)
+    z, _ = TO.forward(desc, geom, x, False)
+    gf = TO.input_gradient(z, x, TO.dz_ce(z, y.view(1, -1), 1.0 / 1024))
+    rel_f = ((gf[:, :3] - go[:, :3]).norm() / go[:, :3].norm()).item()
+    print(f"{arch}: plain vs oracle logp {err:.2e} grad rel {rel:.2e} (xyz {rel_xyz:.2e}, features-only walk "
+          f"{rel_f:.2e}) | tf32 vs oracle logp {err1:.2e} grad rel {rel1:.2e}")
     # what is left is the BatchNorm folding, whose weights describe() stores in fp32
-    assert err < 1e-4 and rel < 1e-4
+    assert err < 1e-4 and rel < 1e-4 and rel_xyz < 1e-4
+    assert rel_f > 1e-2
     assert 1e-3 < err1 < 0.5 and 1e-3 < rel1 < 0.5
 
 
@@ -165,98 +171,15 @@ def _model(arch):
     return _MODELS[arch]
 
 
-def _prof_counts():
-    from pointsecguard_b200 import _lib as L
-    n = L.psg_prof_ncat()
-    ms, cnt = (C.c_double * n)(), (C.c_int64 * n)()
-    assert L.psg_prof_collect(ms, cnt) == 0
-    return {L.psg_prof_name(i).decode(): int(cnt[i]) for i in range(n)}
-
-
-def _grad_stats(mine, ref):
-    mine, ref = mine.double(), ref.double()
-    rel = ((mine - ref).norm() / ref.norm()).item()
-    nz = ref != 0
-    sign = (torch.sign(mine[nz]) == torch.sign(ref[nz])).double().mean().item()
-    close = ((mine - ref).abs() <= 1e-3 * ref.abs() + 1e-12).double().mean().item()
-    return rel, sign, close
-
-
-def _inputs(B, kind, seed=0):
-    x = syn.make_blocks(B, N, seed, kind)
-    lab = syn.zband_labels(x).to(torch.int32).view(-1)
-    dlogp = torch.randn(B, N, 13, generator=torch.Generator().manual_seed(seed + 1)) / N
-    return x.cuda(), lab.cuda(), dlogp.cuda()
-
-
-KAPPA = 0.2
-
-
 def _run_engine(arch, B, kind, mode, sa_compact=1):
-    """Forward, the three loss kinds and the backward on a fresh engine; each loss once after forward(want_logp=True)
-    and once after forward(want_logp=False) (the deferred fp1 + head pass).  Returns the outputs, the launch counts of
-    the first forward + backward, the geometry and the inputs."""
-    from pointsecguard_b200 import _lib as L
-    from pointsecguard_b200.engine import Engine
     desc = _model(arch).describe()
-    eng = Engine(desc, torch.device("cuda", 0), mode)
-    x, lab, dlogp = _inputs(B, kind)
-    out = {}
-    L.psg_set_option(b"sa_compact", sa_compact)
-    try:
-        eng.bind(B, N, 1)
-        eng.set_input(x)
-        torch.manual_seed(0)
-        eng.geometry(eng.draw_starts(1))
-        losses = {0: lambda: eng.loss_grad_generic(dlogp), 1: lambda: eng.loss_grad_ce(lab, -1, 1.0 / N),
-                  2: lambda: eng.loss_grad_cw(lab, -1, 1.0, KAPPA)}
-        _prof_counts()
-        L.psg_prof_enable(1)
-        try:
-            out["logp"], out["l4"] = eng.forward(0, True, True)
-            losses[0]()
-            out[(0, True)] = eng.backward(0)
-            counts = _prof_counts()
-        finally:
-            L.psg_prof_enable(0)
-        for k in (1, 2):
-            eng.forward(0, True, False)
-            losses[k]()
-            out[(k, True)] = eng.backward(0)
-        for k in (0, 1, 2):
-            eng.forward(0, False, False)
-            losses[k]()
-            out[(k, False)] = eng.backward(0)
-        geom = TO.read_engine_geometry(eng)
-        torch.cuda.synchronize()
-    finally:
-        L.psg_set_option(b"sa_compact", 1)
-    return out, counts, geom, desc, (x, lab, dlogp)
-
-
-def _reference(desc, geom, inputs, tf32):
-    x0, lab, dlogp = inputs
-    B = x0.shape[0]
-    x = x0.double().requires_grad_(True)
-    z, l4 = TO.forward(desc, geom, x, tf32)
-    lab2 = lab.view(B, N)
-    dz = {0: TO.dz_generic(z, dlogp.double()), 1: TO.dz_ce(z, lab2, 1.0 / N), 2: TO.dz_cw(z, lab2, 1.0, KAPPA)}
-    res = {"logp": torch.log_softmax(z, -1).detach(), "l4": l4.detach()}
-    for k in (0, 1, 2):
-        res[k] = TO.input_gradient(z, x, dz[k].detach(), retain_graph=k < 2)
-    return res
+    inputs = TO.engine_inputs(B, N, kind)
+    out, counts, geom = TO.run_engine(desc, inputs, mode, sa_compact)
+    return out, counts, geom, desc, inputs
 
 
 def _compare(out, ref, arch, B, what):
-    lp = (out["logp"].double() - ref["logp"]).abs().max().item()
-    l4 = ((out["l4"].double() - ref["l4"]).abs().max() / ref["l4"].abs().max()).item()
-    grads = {key: _grad_stats(out[key], ref[key[0]]) for key in out if isinstance(key, tuple)}
-    worst = (max(g[0] for g in grads.values()), min(g[1] for g in grads.values()), min(g[2] for g in grads.values()))
-    print(f"{arch} B={B} vs {what}: logp {lp:.2e} l4 {l4:.2e} grad rel {worst[0]:.2e} sign {worst[1]:.6f} "
-          f"within-rtol-1e-3 {worst[2]:.5f}")
-    for key, g in sorted(grads.items()):
-        print(f"    loss kind {key[0]} want_logp={key[1]}: rel {g[0]:.2e} sign {g[1]:.6f} close {g[2]:.5f}")
-    return lp, l4, worst
+    return TO.compare(out, ref, f"{arch} B={B}", what)
 
 
 # (arch, B, cloud kind, sa_compact): fp2 (B * 1024 rows) is a tile program from 48 row tiles on, i.e. B >= 6, fp3
@@ -286,9 +209,9 @@ def test_tf32_network_vs_tf32_exact_reference(case):
     got = {k: counts[k] for k in want}
     print(f"{arch} B={B} {kind} compact={compact}: launches {got}")
     assert got == want
-    exact = _reference(desc, geom, inputs, tf32=True)
+    exact = TO.reference(desc, geom, inputs, tf32=True)
     lp, l4, (rel, sign, _) = _compare(out, exact, arch, B, "TF32-exact")
-    plain = _reference(desc, geom, inputs, tf32=False)
+    plain = TO.reference(desc, geom, inputs, tf32=False)
     lp0, _, (rel0, _, _) = _compare(out, plain, arch, B, "plain fp64")
     assert lp < LOGP_GATE and l4 < L4_GATE
     assert rel < GRAD_REL_GATE and sign >= SIGN_GATE
@@ -307,7 +230,7 @@ def test_fp32_grade_modes_vs_plain_reference(case):
     against the plain fp64 reference through the same walk (gates: FP32_* above)."""
     mode, arch, B, kind = case
     out, _, geom, desc, inputs = _run_engine(arch, B, kind, mode)
-    plain = _reference(desc, geom, inputs, tf32=False)
+    plain = TO.reference(desc, geom, inputs, tf32=False)
     lp, l4, (rel, sign, _) = _compare(out, plain, arch, B, f"plain fp64 (mode {mode})")
     assert lp < FP32_LOGP_ATOL and l4 < 1e-4
     assert rel < FP32_GRAD_REL and sign >= FP32_SIGN
