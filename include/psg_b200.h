@@ -57,9 +57,13 @@ int psg_ball_query(const float *xyz, int nclouds, int P, int N, const float *new
                    const double *radius_host, const int *nsample_host, int32_t *out0, int32_t *out1,
                    psg_stream_t stream);
 
-/* Same results through a uniform grid over the cloud (cell edge >= 1.01 r): a centroid tests only the
- * points of its 27 neighbouring cells and emits the hits smallest index first; centroids with more than
- * 96 hits fall back to the exhaustive scan.  ~8x less work than the scan at SA1 densities. */
+/* Same results as psg_ball_query for every input, bit for bit, through a uniform grid over the cloud
+ * (cell edge >= 1.01 r): a centroid tests only the points of its 27 neighbouring cells and emits the hits
+ * smallest index first.  A centroid takes the exhaustive scan instead when it has more than 96 hits, or
+ * when the distance formula's rounding error, which grows with |q|^2 + max|p|^2, is not proven to stay
+ * inside cell^2 - r^2 (clouds far from the origin; the rule is in csrc/ballgrid.cu).  A cloud with a
+ * non-finite coordinate is scanned for every centroid, so a NaN distance counts as a hit, as the
+ * reference counts it.  ~8x less work than the scan at SA1 densities near the origin. */
 size_t psg_ball_grid_workspace(int nclouds, int N);
 int psg_ball_query_grid(const float *xyz, int nclouds, int P, int N, const float *new_xyz, int S, int nr,
                         const double *radius_host, const int *nsample_host, int32_t *out0, int32_t *out1,

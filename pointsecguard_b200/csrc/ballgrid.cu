@@ -8,9 +8,26 @@
 // evaluations per SA1 cloud, ~5 hits each -- the largest item of the per-step geometry cost.  Here the
 // cloud is binned once into cells of edge >= 1.01 r (+1e-4), a centroid only tests the points of its
 // 27 neighbouring cells (the membership test is per pair, so using the same oracle-exact formula on a
-// superset of the hits gives bit-identical membership; the formula's error, ~1e-6 in d2, is far inside
-// the cell margin), and the hits -- found in cell order -- are emitted smallest index first.  A
-// centroid with more hits than the per-warp list holds falls back to the exhaustive scan.
+// superset of the hits gives bit-identical membership), and the hits -- found in cell order -- are
+// emitted smallest index first.  A centroid with more hits than the per-warp list holds falls back to
+// the exhaustive scan.
+//
+// The superset holds only while the formula's rounding error stays below the cell margin cell^2 - r^2,
+// and that error grows with the coordinates, not with r.  With u = 2^-24, Q = |q|^2 (centroid), P = |p|^2
+// (point) and M = max |p|^2 over the cloud: psg_sqdist's dot (one multiply, two FMAs) is within 3u |q||p|,
+// |q|^2 and |p|^2 (three roundings each) within 3u Q and 3u P, and the two rounded adds add u (2Q + P)
+// and u d2, so the computed d2 is within 8u (Q + P) + u d2 of |q - p|^2.  Cell indices are rounded too
+// ((x - min) * inv_cell: three roundings, plus the clamp of the last cell), so a point outside the 27
+// cells may lie up to 3u (|q| + 5 sqrt(M)) nearer than one cell edge along the separating axis; squared,
+// that costs at most 3u Q + 15u M + 18u cell^2.  Such a point cannot be a hit when
+// 23u (Q + M) + 19u cell^2 < cell^2 - r^2.  ball_grid_kernel requires the stronger
+//     2^-19 (Q + M + cell^2) < cell^2 - r^2          (2^-19 = 32u: 1.4x the bound, covering the test's own rounding)
+// and sends every other centroid straight to the exhaustive scan.  At r = 0.1 (cell 0.1011) that admits
+// Q + M < 116 m^2, and even an ungrown cell at r = 0.05 (0.0506) admits Q + M < 31 m^2, so a 1 x 1 x 3 m block
+// at the origin (Q + M <= 19) keeps the grid for every centroid; a cloud tens of metres from the origin scans
+// unless its cell grew large (a scene-sized slab).  A cloud with a non-finite coordinate, or whose M
+// overflows, is not binned at all and every centroid scans, so a NaN distance counts as a hit exactly as
+// the reference counts it (!(d > r^2)).
 #include "psg_common.cuh"
 #include "psg_internal.h"
 
@@ -23,6 +40,8 @@ constexpr int kWarps = 8;
 struct GridHdr {
     float minx, miny, minz, inv_cell;
     int gx, gy, gz, ncells;
+    float cell, m2;         // cell edge, max |p|^2 of the cloud
+    int finite;             // 0: a coordinate or an |p|^2 is not finite -- the cloud was not binned, every centroid scans
 };
 
 __host__ __device__ inline size_t grid_bytes_per_cloud(int N)
@@ -56,16 +75,22 @@ __device__ __forceinline__ int cell_of(const GridHdr &h, float x, float y, float
 __global__ void __launch_bounds__(1024) grid_build_kernel(const float *__restrict__ xyz, long long cloud_stride, int N,
                                                           float rmax, unsigned char *__restrict__ ws_all, size_t ws_stride)
 {
-    __shared__ float red[6][32];
+    __shared__ float red[7][32];
     __shared__ GridHdr hdr;
     __shared__ int wsum[32];
     __shared__ int carry_s;
     const float *cloud = xyz + (long long)blockIdx.x * cloud_stride;
     unsigned char *ws = ws_all + (size_t)blockIdx.x * ws_stride;
     const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
-    float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
-    for (int i = t; i < N; i += blockDim.x)
-        for (int a = 0; a < 3; ++a) { const float v = cloud[3 * i + a]; lo[a] = fminf(lo[a], v); hi[a] = fmaxf(hi[a], v); }
+    float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY}, m2 = 0.f;
+    bool fin = true;
+    for (int i = t; i < N; i += blockDim.x) {
+        const float x = cloud[3 * i], y = cloud[3 * i + 1], z = cloud[3 * i + 2];
+        lo[0] = fminf(lo[0], x); lo[1] = fminf(lo[1], y); lo[2] = fminf(lo[2], z);
+        hi[0] = fmaxf(hi[0], x); hi[1] = fmaxf(hi[1], y); hi[2] = fmaxf(hi[2], z);
+        m2 = fmaxf(m2, psg_sqnorm(x, y, z));
+        fin = fin && isfinite(x) && isfinite(y) && isfinite(z);     // fminf / fmaxf skip a NaN: count it here
+    }
     for (int a = 0; a < 3; ++a) {
         for (int o = 16; o > 0; o >>= 1) {
             lo[a] = fminf(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
@@ -73,27 +98,35 @@ __global__ void __launch_bounds__(1024) grid_build_kernel(const float *__restric
         }
         if (lane == 0) { red[a][warp] = lo[a]; red[3 + a][warp] = hi[a]; }
     }
-    __syncthreads();
+    for (int o = 16; o > 0; o >>= 1) m2 = fmaxf(m2, __shfl_xor_sync(0xffffffffu, m2, o));
+    if (lane == 0) red[6][warp] = m2;
+    const bool all_finite = __syncthreads_and(fin);
     if (t == 0) {
-        float l[3], h[3];
+        float l[3], h[3], mm = red[6][0];
         for (int a = 0; a < 3; ++a) {
             l[a] = red[a][0]; h[a] = red[3 + a][0];
             for (int w = 1; w < (int)(blockDim.x >> 5); ++w) { l[a] = fminf(l[a], red[a][w]); h[a] = fmaxf(h[a], red[3 + a][w]); }
         }
-        float cell = rmax * 1.01f + 1e-4f;
-        int gx, gy, gz;
-        for (;;) {
-            gx = (int)floorf((h[0] - l[0]) / cell) + 1; gy = (int)floorf((h[1] - l[1]) / cell) + 1;
-            gz = (int)floorf((h[2] - l[2]) / cell) + 1;
-            if ((long long)gx * gy * gz <= kMaxCells) break;
-            cell *= 1.26f;                       // ~ halves the cell count
+        for (int w = 1; w < (int)(blockDim.x >> 5); ++w) mm = fmaxf(mm, red[6][w]);
+        // finite coordinates with a finite max |p|^2 bound every extent below 4e19: the cell counts below stay finite
+        hdr.finite = all_finite && mm < INFINITY;
+        float cell = rmax * 1.01f + 1e-4f, fx = 1.f, fy = 1.f, fz = 1.f;
+        if (hdr.finite) {
+            for (;;) {                           // counted in float: an extent of 2^31 cells must not wrap an int
+                fx = floorf((h[0] - l[0]) / cell) + 1.f; fy = floorf((h[1] - l[1]) / cell) + 1.f;
+                fz = floorf((h[2] - l[2]) / cell) + 1.f;
+                if ((double)fx * fy * fz <= kMaxCells) break;
+                cell *= 1.26f;                   // ~ halves the cell count
+            }
         }
         hdr.minx = l[0]; hdr.miny = l[1]; hdr.minz = l[2]; hdr.inv_cell = 1.0f / cell;
-        hdr.gx = gx; hdr.gy = gy; hdr.gz = gz; hdr.ncells = gx * gy * gz;
+        hdr.gx = (int)fx; hdr.gy = (int)fy; hdr.gz = (int)fz; hdr.ncells = hdr.gx * hdr.gy * hdr.gz;
+        hdr.cell = cell; hdr.m2 = mm;
         *g_hdr(ws) = hdr;
         carry_s = 0;
     }
     __syncthreads();
+    if (!hdr.finite) return;                     // not binned: ball_grid_kernel scans every centroid of this cloud
     int *start = g_start(ws), *cursor = g_cursor(ws);
     const int nc = hdr.ncells;
     for (int c = t; c <= nc; c += blockDim.x) start[c] = 0;
@@ -185,13 +218,16 @@ ball_grid_kernel(const unsigned char *__restrict__ ws_all, size_t ws_stride, con
     const int kmax = 0x7fffffff;
     int a0 = kmax, a1 = kmax, a2 = kmax, b0 = kmax, b1 = kmax, b2 = kmax;   // hit lists, 3 slots per lane
     int cnta = 0, cntb = 0;
-    bool overflow = false;
+    // the margin rule of the file comment: the 27 cells hold every hit only when the rounding error of the distance
+    // formula is proven to stay inside cell^2 - r^2 (false for a NaN centroid and for a cloud that was not binned)
+    const float r2max = NR == 2 ? fmaxf(r2a, r2b) : r2a;
+    bool scan = !h.finite || !(0x1p-19f * ((qn + h.m2) + h.cell * h.cell) < h.cell * h.cell - r2max);
     int cx = (int)floorf((qx - h.minx) * h.inv_cell), cy = (int)floorf((qy - h.miny) * h.inv_cell),
         cz = (int)floorf((qz - h.minz) * h.inv_cell);
-    for (int dz = -1; dz <= 1 && !overflow; ++dz) {
+    for (int dz = -1; dz <= 1 && !scan; ++dz) {
         const int z = cz + dz;
         if (z < 0 || z >= h.gz) continue;
-        for (int dy = -1; dy <= 1 && !overflow; ++dy) {
+        for (int dy = -1; dy <= 1 && !scan; ++dy) {
             const int y = cy + dy;
             if (y < 0 || y >= h.gy) continue;
             // the three x-neighbours are consecutive cells: one contiguous range of sorted points
@@ -212,16 +248,16 @@ ball_grid_kernel(const unsigned char *__restrict__ ws_all, size_t ws_stride, con
                 }
                 push_hits(__ballot_sync(0xffffffffu, ha), id, lane, cnta, a0, a1, a2);
                 if (NR == 2) push_hits(__ballot_sync(0xffffffffu, hb), id, lane, cntb, b0, b1, b2);
-                if (cnta > kCap || cntb > kCap) { overflow = true; break; }
+                if (cnta > kCap || cntb > kCap) { scan = true; break; }
             }
         }
     }
-    if (!overflow) {
+    if (!scan) {
         emit_sorted(a0, a1, a2, cnta, Ka, N, oa, lane);
         if (NR == 2) emit_sorted(b0, b1, b2, cntb, Kb, N, ob, lane);
         return;
     }
-    // ---- fallback: exhaustive scan in index order (dense neighbourhoods) ----
+    // ---- fallback: exhaustive scan in index order (dense neighbourhoods; centroids outside the margin rule) ----
     const float *cloud = xyz + (long long)cloud_id * cloud_stride;
     cnta = cntb = 0;
     int firsta = -1, firstb = -1;

@@ -207,9 +207,14 @@ three_nn_grid_kernel(const float *__restrict__ xyz1, long long stride1, int nclo
 
     // ---- bounding box of the coarse cloud ----
     float mn[3] = {INFINITY, INFINITY, INFINITY}, mx[3] = {-INFINITY, -INFINITY, -INFINITY};
+    bool fin = true;
     for (int j = t; j < S; j += 256) {
 #pragma unroll
-        for (int a = 0; a < 3; ++a) { const float v = coarse[3 * j + a]; mn[a] = fminf(mn[a], v); mx[a] = fmaxf(mx[a], v); }
+        for (int a = 0; a < 3; ++a) {
+            const float v = coarse[3 * j + a];
+            mn[a] = fminf(mn[a], v); mx[a] = fmaxf(mx[a], v);
+            fin = fin && isfinite(v);                                // fminf / fmaxf skip a NaN: count it here
+        }
     }
 #pragma unroll
     for (int a = 0; a < 3; ++a) {
@@ -220,7 +225,7 @@ three_nn_grid_kernel(const float *__restrict__ xyz1, long long stride1, int nclo
         }
         if (lane == 0) { red[a][warp] = mn[a]; red[3 + a][warp] = mx[a]; }
     }
-    __syncthreads();
+    const bool all_finite = __syncthreads_and(fin);
     if (t == 0) {
         float lo[3], hi[3], ext[3];
         for (int a = 0; a < 3; ++a) {
@@ -236,6 +241,7 @@ three_nn_grid_kernel(const float *__restrict__ xyz1, long long stride1, int nclo
         while (d[0] * d[1] * d[2] > kNgMaxCells) { h *= 1.26f; for (int a = 0; a < 3; ++a) { d[a] = (int)(ext[a] / h) + 1; d[a] = d[a] > 16 ? 16 : d[a]; } }
         float m2 = 0.f;
         for (int a = 0; a < 3; ++a) { const float v = fmaxf(fabsf(lo[a]), fabsf(hi[a])); m2 += v * v; }
+        if (!all_finite) m2 = INFINITY;                                  // every query scans (below)
         sb[0] = lo[0]; sb[1] = lo[1]; sb[2] = lo[2]; sb[3] = h; sb[4] = m2;            // m2 >= |p|^2 of every coarse point
         sdim[0] = d[0]; sdim[1] = d[1]; sdim[2] = d[2]; sdim[3] = d[0] * d[1] * d[2];
     }
@@ -283,13 +289,21 @@ three_nn_grid_kernel(const float *__restrict__ xyz1, long long stride1, int nclo
     for (int qi = q0 + t; qi < min(q0 + kNgQ, N); qi += 256) {
         const float qx = fine[3 * qi], qy = fine[3 * qi + 1], qz = fine[3 * qi + 2];
         const float qn = psg_sqnorm(qx, qy, qz);
+        float d0 = INFINITY, d1 = INFINITY, d2 = INFINITY;
+        int i0 = -1, i1 = -1, i2 = -1;
+        // A non-finite query or coarse cloud, or an |p|^2 that overflows, can make distances NaN, which the (distance,
+        // index) order cannot rank: such a query scans every coarse point in index order with three_nn_kernel's
+        // insertion, so it returns what the exhaustive kernel returns for any input.
+        const bool scan = !(qn < INFINITY && m2c < INFINITY);
+        for (int j = 0; scan && j < S; ++j) {
+            const float x = coarse[3 * j], y = coarse[3 * j + 1], z = coarse[3 * j + 2];
+            top3_push(psg_sqdist(qx, qy, qz, qn, x, y, z, psg_sqnorm(x, y, z)), j, d0, d1, d2, i0, i1, i2);
+        }
         // rounding error of the expansion formula <= ~2.4e-6 * max(|q|^2, |p|^2): a 16x safety factor
         const float margin = 4e-5f * (1.0f + fmaxf(qn, m2c));
         int cx, cy, cz;
         cell_of(qx, qy, qz, cx, cy, cz);
-        float d0 = INFINITY, d1 = INFINITY, d2 = INFINITY;
-        int i0 = -1, i1 = -1, i2 = -1;
-        const int rmax = max(max(max(cx, nx - 1 - cx), max(cy, ny - 1 - cy)), max(cz, nz - 1 - cz));
+        const int rmax = scan ? -1 : max(max(max(cx, nx - 1 - cx), max(cy, ny - 1 - cy)), max(cz, nz - 1 - cz));
         for (int r = 0; r <= rmax; ++r) {
             for (int dz = -r; dz <= r; ++dz) {
                 const int z = cz + dz;
