@@ -240,6 +240,15 @@ int psg_net_pgd_update(psg_net *net, float *adv, const float *ori, const uint8_t
  * have been built; labels int32 [B,N] (kind-1 loss), target < 0 for the non-targeted attack. */
 int psg_nb_attack(psg_net *net, float *adv, const float *ori, const uint8_t *mask, const int32_t *labels,
                   int target, int iters, int t0, float alpha, float eps, float scale, psg_stream_t stream);
+/* L2-ball variants of the two calls above (torchattacks PGDL2), same arguments.  Per block b, over the moving points of
+ * the field (all, or mask != 0): a = cur + alpha_signed * g / (||g||_2 + 1e-10) is written to adv (un-projected), and
+ * ori + (a - ori) * min(eps / ||a - ori||_2, 1), clamped to [lo, hi], becomes the next model input.  The norms are fp32
+ * square roots of double sums in a fixed order: a block's result does not depend on the other blocks of the batch.
+ * PSG_EINVAL for a bad field, eps < 0 or a non-finite alpha / eps. */
+int psg_net_pgd_update_l2(psg_net *net, float *adv, const float *ori, const uint8_t *mask, int c0, int nc,
+                          float alpha_signed, float eps, float lo, float hi, psg_stream_t stream);
+int psg_nb_attack_l2(psg_net *net, float *adv, const float *ori, const uint8_t *mask, const int32_t *labels,
+                     int target, int iters, int t0, float alpha, float eps, float scale, psg_stream_t stream);
 /* ---- norm-unbounded attacks: NU_attack (nontarget.py:52-106), tar_NU_attack (target.py:62-133) ----
  * All buffers are caller-owned device memory.  One psg_nu_step enqueues, with no host round trip:
  * colours = (tanh(w)+1)/2 written into the model input and `adv`; forward t; C&W f and its gradient

@@ -104,6 +104,8 @@ _PROTOS = {
     "psg_net_backward": (_i, [_vp, _i, _vp, _vp]),
     "psg_net_pgd_update": (_i, [_vp, _vp, _vp, _vp, _i, _i, _f, _f, _f, _f, _vp]),
     "psg_nb_attack": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _f, _f, _f, _vp]),
+    "psg_net_pgd_update_l2": (_i, [_vp, _vp, _vp, _vp, _i, _i, _f, _f, _f, _f, _vp]),
+    "psg_nb_attack_l2": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _f, _f, _f, _vp]),
     "psg_nu_scratch_floats": (_sz, [_i, _i]),
     "psg_nu_init": (_i, [_vp, C.POINTER(NuBuffers), _vp]),
     "psg_nu_step": (_i, [_vp, C.POINTER(NuBuffers), _i, _i, _i, _i, _f, _f, _f, _f, _f, _i, _d, _d, _i, _i, _vp, _vp]),

@@ -105,6 +105,77 @@ __global__ void pgd_update_kernel(float *__restrict__ adv, const float *__restri
     }
 }
 
+// L2-ball variant of the step above (torchattacks PGDL2), one CTA per block b over its moving points (all, or the masked):
+//   gn = fp32(sqrt(sum double(g)^2));  a = cur + alpha_signed * (g / (gn + 1e-10f))  -> adv (un-projected, as above)
+//   d = a - ori;  dn = fp32(sqrt(sum double(d)^2));  f = dn > eps ? eps / dn : 1;  col = clamp(ori + d * f, lo, hi) -> feats0
+// Every element op is separately rounded fp32.  The sums are per-thread partials in a fixed point order, a fixed shuffle
+// tree and a warp-order pass, so a block's result depends on N and its own data only (not on B, sharding or chunking).
+constexpr int kL2Threads = 512;
+
+__device__ __forceinline__ double l2_block_sum(double v, double *sh)
+{
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = __dadd_rn(v, __shfl_xor_sync(0xffffffffu, v, o));
+    if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = v;
+    __syncthreads();
+    double s = 0.0;
+#pragma unroll
+    for (int w = 0; w < kL2Threads / 32; ++w) s = __dadd_rn(s, sh[w]);
+    __syncthreads();                                               // sh is reused by the next sum
+    return s;
+}
+
+__global__ void __launch_bounds__(kL2Threads) pgd_l2_update_kernel(float *__restrict__ adv, const float *__restrict__ ori,
+                                                                  TView grad, TView feats0,
+                                                                  const unsigned char *__restrict__ mask, int C, int N,
+                                                                  int c0, int nc, float alpha_signed, float eps, float lo,
+                                                                  float hi)
+{
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    asm volatile("griddepcontrol.wait;" ::: "memory");          // launched with programmatic stream serialization
+    __shared__ double sh[kL2Threads / 32];
+    const int b = blockIdx.x;
+    const long long row0 = (long long)b * N;
+    const unsigned char *mk = mask ? mask + row0 : nullptr;
+    auto g_at = [&](int n, int ch) { return grad.base[tv_off(grad, row0 + n, ch >> 2) + (ch & 3)]; };
+    auto f_at = [&](int n, int ch) { return feats0.base + tv_off(feats0, row0 + n, ch >> 2) + (ch & 3); };
+
+    double s = 0.0;                                                // pass 1: sum g^2
+    for (int n = threadIdx.x; n < N; n += kL2Threads) {
+        if (mk && mk[n] == 0) continue;
+        for (int j = 0; j < nc; ++j) {
+            const double g = g_at(n, c0 + j);
+            s = __dadd_rn(s, __dmul_rn(g, g));
+        }
+    }
+    const float den = __fadd_rn(__double2float_rn(sqrt(l2_block_sum(s, sh))), 1e-10f);
+
+    s = 0.0;                                                       // pass 2: write adv, sum d^2
+    for (int n = threadIdx.x; n < N; n += kL2Threads) {
+        if (mk && mk[n] == 0) continue;
+        for (int j = 0; j < nc; ++j) {
+            const int ch = c0 + j;
+            const float a = __fadd_rn(*f_at(n, ch), __fmul_rn(alpha_signed, __fdiv_rn(g_at(n, ch), den)));
+            adv[((long long)b * C + ch) * N + n] = a;
+            const double d = __fsub_rn(a, ori[((long long)b * nc + j) * N + n]);
+            s = __dadd_rn(s, __dmul_rn(d, d));
+        }
+    }
+    const float dn = __double2float_rn(sqrt(l2_block_sum(s, sh)));
+    const float f = dn > eps ? __fdiv_rn(eps, dn) : 1.f;
+
+    for (int n = threadIdx.x; n < N; n += kL2Threads) {            // pass 3: the same a and d, projected and clamped
+        if (mk && mk[n] == 0) continue;
+        for (int j = 0; j < nc; ++j) {
+            const int ch = c0 + j;
+            float *fp = f_at(n, ch);
+            const float a = __fadd_rn(*fp, __fmul_rn(alpha_signed, __fdiv_rn(g_at(n, ch), den)));
+            const float o = ori[((long long)b * nc + j) * N + n];
+            *fp = fminf(fmaxf(__fadd_rn(o, __fmul_rn(__fsub_rn(a, o), f)), lo), hi);
+        }
+    }
+}
+
 // conf[label][pred] += 1 with pred = first arg-max of the log-probabilities, followed by four
 // scalars: rows seen, rows with pred == label, masked rows, masked rows with pred == target
 __global__ void confusion_kernel(const float *__restrict__ logp, const int *__restrict__ labels,
@@ -190,6 +261,14 @@ int psg_pgd_update(float *adv, const float *ori, TView grad, TView feats0, const
 {
     if (psg_launch_pdl(pgd_update_kernel, dim3(nb((long long)B * N, 256)), dim3(256), 0, st, 1, adv, ori, grad, feats0, mask, B, C, N, c0,
                        nc, alpha_signed, eps, lo, hi) != cudaSuccess) return PSG_ECUDA;
+    PSG_LAUNCH_CHECK();
+    return PSG_OK;
+}
+int psg_pgd_l2_update(float *adv, const float *ori, TView grad, TView feats0, const unsigned char *mask, int B, int C,
+                      int N, int c0, int nc, float alpha_signed, float eps, float lo, float hi, cudaStream_t st)
+{
+    if (psg_launch_pdl(pgd_l2_update_kernel, dim3((unsigned)B), dim3(kL2Threads), 0, st, 1, adv, ori, grad, feats0, mask, C,
+                       N, c0, nc, alpha_signed, eps, lo, hi) != cudaSuccess) return PSG_ECUDA;
     PSG_LAUNCH_CHECK();
     return PSG_OK;
 }

@@ -13,6 +13,7 @@
 //   * Activations live in T-layout (psg_common.cuh); every conv(1x1)+BN(eval)+ReLU is one GEMM with
 //     the BN folded into W,b; FP concat is a two-source A operand; dgrad only, no wgrad.
 //   * No allocation, no synchronisation, no host round trip inside forward / backward / attack.
+#include <cmath>
 #include <cstring>
 #include <new>
 #include <vector>
@@ -1089,10 +1090,25 @@ extern "C" int psg_net_pgd_update(psg_net *n, float *adv, const float *ori, cons
     return PSG_OK;
 }
 
-extern "C" int psg_nb_attack(psg_net *n, float *adv, const float *ori, const uint8_t *mask, const int32_t *labels,
-                             int target, int iters, int t0, float alpha, float eps, float scale, psg_stream_t stream)
+// torchattacks PGDL2's step and projection on the same field (elementwise.cu, pgd_l2_update_kernel): the norms are taken
+// per block over its moving points, so eps is an L2 radius in colour space
+extern "C" int psg_net_pgd_update_l2(psg_net *n, float *adv, const float *ori, const uint8_t *mask, int c0, int nc,
+                                     float alpha_signed, float eps, float lo, float hi, psg_stream_t stream)
+{
+    if (!n || !n->bound || !adv || !ori || c0 < 0 || nc <= 0 || c0 + nc > n->in_channels) return PSG_EINVAL;
+    if (!std::isfinite(alpha_signed) || !std::isfinite(eps) || eps < 0.f) return PSG_EINVAL;
+    cudaStream_t st = (cudaStream_t)stream;
+    PSG_RUN(PF_PGD, psg_pgd_l2_update(adv, ori, tv(n->dfeat[0], n->wfeat[0]), tv(n->feats[0], n->wfeat[0]), mask, n->B,
+                                      n->in_channels, n->N, c0, nc, alpha_signed, eps, lo, hi, st));
+    return PSG_OK;
+}
+
+// The NB / tar-NB loop body shared by both norms: forward, cross-entropy gradient, backward, update on colours 3:6.
+static int nb_loop(psg_net *n, bool l2, float *adv, const float *ori, const uint8_t *mask, const int32_t *labels, int target,
+                   int iters, int t0, float alpha, float eps, float scale, psg_stream_t stream)
 {
     if (!n || !n->bound || iters < 0 || t0 < 0 || t0 + iters > n->T) return PSG_EINVAL;
+    if (l2 && (!std::isfinite(alpha) || !std::isfinite(eps) || eps < 0.f)) return PSG_EINVAL;
     // non-targeted: ascent on the true-label cost (nontarget.py:37); targeted: descent on the
     // target-label cost (target.py:41)
     const float a = target >= 0 ? -alpha : alpha;
@@ -1100,9 +1116,22 @@ extern "C" int psg_nb_attack(psg_net *n, float *adv, const float *ori, const uin
         PSG_TRY(psg_net_forward(n, t0 + i, nullptr, nullptr, stream));
         PSG_TRY(psg_net_loss_grad(n, 1, nullptr, labels, target, scale, 0.f, nullptr, stream));
         PSG_TRY(psg_net_backward(n, t0 + i, nullptr, stream));
-        PSG_TRY(psg_net_pgd_update(n, adv, ori, mask, 3, 3, a, eps, 0.f, 1.f, stream));
+        PSG_TRY(l2 ? psg_net_pgd_update_l2(n, adv, ori, mask, 3, 3, a, eps, 0.f, 1.f, stream)
+                   : psg_net_pgd_update(n, adv, ori, mask, 3, 3, a, eps, 0.f, 1.f, stream));
     }
     return PSG_OK;
+}
+
+extern "C" int psg_nb_attack(psg_net *n, float *adv, const float *ori, const uint8_t *mask, const int32_t *labels,
+                             int target, int iters, int t0, float alpha, float eps, float scale, psg_stream_t stream)
+{
+    return nb_loop(n, false, adv, ori, mask, labels, target, iters, t0, alpha, eps, scale, stream);
+}
+
+extern "C" int psg_nb_attack_l2(psg_net *n, float *adv, const float *ori, const uint8_t *mask, const int32_t *labels,
+                                int target, int iters, int t0, float alpha, float eps, float scale, psg_stream_t stream)
+{
+    return nb_loop(n, true, adv, ori, mask, labels, target, iters, t0, alpha, eps, scale, stream);
 }
 
 // ------------------------------------------------------------------------------------------------

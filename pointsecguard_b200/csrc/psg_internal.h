@@ -173,6 +173,8 @@ int psg_dz_cw(TView z, const int *labels, int target, long long rows, int ncls, 
               float *loss_rows, unsigned char *hit, cudaStream_t st);
 int psg_pgd_update(float *adv, const float *ori, TView grad, TView feats0, const unsigned char *mask, int B, int C,
                    int N, int c0, int nc, float alpha_signed, float eps, float lo, float hi, cudaStream_t st);
+int psg_pgd_l2_update(float *adv, const float *ori, TView grad, TView feats0, const unsigned char *mask, int B, int C,
+                      int N, int c0, int nc, float alpha_signed, float eps, float lo, float hi, cudaStream_t st);
 int psg_confusion(const float *logp, const int *labels, const unsigned char *mask, int target, long long rows, int ncls,
                   long long *conf, cudaStream_t st);
 int psg_add_vote_k(const float *logp, const long long *point_idx, const float *weight, long long rows, int ncls, float *pool,

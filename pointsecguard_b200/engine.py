@@ -270,7 +270,16 @@ class Engine:
                              c0, nc, alpha_signed, eps, lo, hi, self._stream())
 
     @_on_engine_device
-    def nb_attack(self, adv, ori, mask, labels, target, iters, t0, alpha, eps, scale):
-        L.psg_nb_attack(self._net, adv.data_ptr(), ori.data_ptr(), mask.data_ptr() if mask is not None else None,
-                        labels.data_ptr() if labels is not None else None, target, iters, t0, alpha, eps, scale,
-                        self._stream())
+    def pgd_update_l2(self, adv, ori, mask, c0, nc, alpha_signed, eps, lo=0.0, hi=1.0):
+        """``pgd_update`` with torchattacks PGDL2's step and L2-ball projection, per block over its moving points."""
+        L.psg_net_pgd_update_l2(self._net, adv.data_ptr(), ori.data_ptr(), mask.data_ptr() if mask is not None else None,
+                                c0, nc, alpha_signed, eps, lo, hi, self._stream())
+
+    @_on_engine_device
+    def nb_attack(self, adv, ori, mask, labels, target, iters, t0, alpha, eps, scale, norm="Linf"):
+        """``iters`` NB / tar-NB iterations from forward slot t0; ``norm`` "Linf" (sign step) or "L2" (PGDL2 step)."""
+        if norm not in ("Linf", "L2"):
+            raise ValueError(f"norm must be 'Linf' or 'L2', got {norm!r}")
+        fn = L.psg_nb_attack if norm == "Linf" else L.psg_nb_attack_l2
+        fn(self._net, adv.data_ptr(), ori.data_ptr(), mask.data_ptr() if mask is not None else None,
+           labels.data_ptr() if labels is not None else None, target, iters, t0, alpha, eps, scale, self._stream())

@@ -1,7 +1,8 @@
 """Non-targeted colour attacks -- drop-in for PointNet/attacks/torchattacks/attacks/nontarget.py.
 
 NB_attack (:10-42): L-inf sign ascent on sum-CE / N over channels 3:6; the returned tensor is the
-un-projected last step (Q1).  The whole loop is one C call (psg_nb_attack): the geometry of all
+un-projected last step (Q1).  ``norm="L2"`` replaces the sign step and box projection by torchattacks PGDL2's
+normalised-gradient step and per-block L2-ball projection (eps is then the radius of the ball).  The whole loop is one C call (psg_nb_attack): the geometry of all
 ``iters`` forwards is computed in one batched pass first, because for a colour attack it depends
 only on xyz and on the FPS start draws (made here on the CPU generator in the reference's order).
 """
@@ -12,14 +13,30 @@ import torch
 from ..attack import Attack
 
 _MAX_PROBLEMS = 1024     # FPS problems (= forwards x blocks) whose geometry is resident at once
+NORMS = ("Linf", "L2")
+
+
+def _check_norm(norm):
+    if norm not in NORMS:
+        raise ValueError(f"norm must be one of {NORMS}, got {norm!r}")
+    return norm
+
+
+def _str_with_norm(s, norm):
+    """The string form of the reference's attacks, with the norm listed when it is not the reference's L-inf."""
+    return s if norm == "Linf" else s[:-1] + f", norm={norm})"
 
 
 class NB_attack(Attack):
-    def __init__(self, model, eps=0.3, alpha=2 / 255, iters=40):
+    def __init__(self, model, eps=0.3, alpha=2 / 255, iters=40, norm="Linf"):
         super().__init__("NB_attack", model)
         self.eps = eps
         self.alpha = alpha
         self.iters = iters
+        self._norm = _check_norm(norm)
+
+    def __str__(self):
+        return _str_with_norm(super().__str__(), self._norm)
 
     def forward(self, images, labels):
         return _nb_loop(self, images, labels, target=-1, mask=None)
@@ -39,8 +56,16 @@ def _nb_loop(atk, images, labels, target, mask):
     dev = images.device
     B, C, N = images.shape
     src = images.detach()
-    # nontarget.py:34: sum-CE / N;  target.py:38: mean CE over the B*N points
-    scale = 1.0 / N if target < 0 else 1.0 / (B * N)
+    norm = atk._norm
+    # nontarget.py:34: sum-CE / N;  target.py:38: mean CE over the B*N points.  The sign step ignores the scale; the L2
+    # step does not (the 1e-10 beside the gradient norm), so there the mean runs over the GLOBAL batch: a shard's blocks
+    # then step exactly as they do in the single-GPU run.
+    if target < 0:
+        scale = 1.0 / N
+    elif norm == "L2":
+        scale = 1.0 / ((eng.shard.global_batch if eng.shard is not None else B) * N)
+    else:
+        scale = 1.0 / (B * N)
     chunk = max(1, min(atk.iters, _MAX_PROBLEMS // B))
     cur = torch.cuda.current_stream()
     eng.use_stream(None)                            # on `cur`: the head start's events order the tail engine against it
@@ -91,16 +116,16 @@ def _nb_loop(atk, images, labels, target, mask):
                 msk[1:] = 0
         if head:
             for i in range(head):
-                eng.nb_attack(adv, ori, msk, lab, target, 1, i, atk.alpha, atk.eps, scale)
+                eng.nb_attack(adv, ori, msk, lab, target, 1, i, atk.alpha, atk.eps, scale, norm)
             cur.wait_event(tail_ready)
             tail.copy_input_from(eng)          # the PROJECTED colours of the head's last update (adv holds the un-projected ones)
             for i in range(t - head):
-                tail.nb_attack(adv, ori, msk, lab, target, 1, i, atk.alpha, atk.eps, scale)
+                tail.nb_attack(adv, ori, msk, lab, target, 1, i, atk.alpha, atk.eps, scale, norm)
             if done + t < atk.iters:
                 eng.copy_input_from(tail)      # the next chunk starts on the primary engine again
         else:
             for i in range(t):
-                eng.nb_attack(adv, ori, msk, lab, target, 1, i, atk.alpha, atk.eps, scale)
+                eng.nb_attack(adv, ori, msk, lab, target, 1, i, atk.alpha, atk.eps, scale, norm)
         done += t
     if adv is None:                                                        # iters == 0
         adv = images.detach().clone(memory_format=torch.contiguous_format)

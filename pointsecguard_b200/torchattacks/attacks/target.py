@@ -4,22 +4,27 @@ tar_NB_attack (:7-45): sign *descent* on the mean CE to ``target`` over all poin
 points' colours move (unmasked points are neither stepped nor clamped, target.py:41-43).  The reference handles
 B == 1 with a [N] mask; handed a batch it still attacks block 0 only (its cost reads ``outputs[0]``, :36), and so does
 this class for a 1-D mask.  A [B,N] mask is the generalisation to batches (SURVEY.md section 8c) with identical
-per-block arithmetic (the step is a sign, so the loss normalisation does not matter).
+per-block arithmetic (the step is a sign, so the loss normalisation does not matter).  ``norm="L2"`` takes torchattacks
+PGDL2's step and per-block L2-ball projection over the masked points instead (nontarget.py, _nb_loop).
 """
 from __future__ import annotations
 
 from ..attack import Attack
-from .nontarget import _nb_loop
+from .nontarget import _check_norm, _nb_loop, _str_with_norm
 
 
 class tar_NB_attack(Attack):
-    def __init__(self, model, eps=0.3, alpha=2 / 255, iters=40, target=None, mask=None):
+    def __init__(self, model, eps=0.3, alpha=2 / 255, iters=40, target=None, mask=None, norm="Linf"):
         super().__init__("tar_NB_attack", model)
         self.eps = eps
         self.alpha = alpha
         self.iters = iters
         self.target = target
         self.mask = mask
+        self._norm = _check_norm(norm)
+
+    def __str__(self):
+        return _str_with_norm(super().__str__(), self._norm)
 
     def forward(self, images, labels):
         if self.target is None or self.mask is None:
